@@ -8,6 +8,7 @@ until the reference's stopping rules fire or maxit = 200 is reached — at 512^3
 value = PARSDMM iterations / second, plain, at every N.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload config3|config2] [--size n] [--impl reference]
+                  [--dump-outputs DIR]
 
 Device arm (default):
   value      problem and m resident in HBM, CUDA-event time of the K solves on the solver stream, max over ranks
@@ -27,6 +28,14 @@ Reference arm (--impl reference): the CPU restatement alone (Julia is not instal
 each step a bounded sample, extrapolated to the full grid by the plane ratio (stated in the line).
 
 Multi-GPU (N>1, torchrun): one process per GPU, z-slabs; peer-memory CG collectives + NCCL (see DESIGN.md §6).
+
+--dump-outputs DIR: after the timed legs, the return value (x, log, l, y) of the last step of the end-to-end leg
+(device arm, one process; the resident leg computes the same projection but leaves x, l, y on the device) or of the
+last CPU sample (reference arm) as DIR/<name>.npy, see output_arrays.  The inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
+
+A run writes nothing into the tree (it may be read-only): the CPU baseline library is built in a temporary
+directory when the tree holds none for this host, and no bytecode is cached.
 """
 from __future__ import annotations
 
@@ -39,6 +48,7 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -69,6 +79,34 @@ def tweak_options(o, maxit=200):
 def relerr(a, b):
     a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
     return float(np.linalg.norm(a - b) / max(np.linalg.norm(b), 1e-300))
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def output_arrays(result):
+    """{name: array} of one PARSDMM return value (x, log, l, y) for --dump-outputs: x, l_<i>, y_<i> and log_<field>
+    for every array of the log (cg_it as float64; evol_x from iteration 2 on: iteration 1 starts from x = 0 with
+    rhs = 0, so its entry is 0/0 = NaN by definition, as in the reference's log).  A vector larger than its share of
+    DUMP_BYTES becomes a sample of its entries at seeded random positions, the same positions for the same arguments.
+    Returns copies: the caller's buffers may be reused."""
+    x, log, l, y = result
+    out = {"log_" + k: np.asarray(v, dtype=np.float64 if v.dtype.kind in "biu" else v.dtype).copy()
+           for k, v in vars(log).items() if isinstance(v, np.ndarray)}
+    out["log_evol_x"] = out["log_evol_x"][1:]
+    vecs = [("x", x)] + [("l_%d" % i, v) for i, v in enumerate(l or [])] + [("y_%d" % i, v) for i, v in enumerate(y or [])]
+    room = DUMP_BYTES - sum(v.nbytes for v in out.values()) - 4096 * (len(out) + len(vecs))       # 4096: .npy header
+    for seed, (name, v) in enumerate(vecs):
+        v = np.asarray(v).ravel()
+        keep = room // len(vecs) // v.itemsize
+        out[name] = v[np.unique(np.random.default_rng(seed).integers(0, v.size, keep))] if v.size > keep else v.copy()
+    return out
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -160,13 +198,13 @@ def cpu_impl():
     if not cpu_threaded_available():
         return "NumPy/SciPy oracle (single-threaded apart from BLAS dot/norm)"
     from oracle import build_c
-    native = build_c.is_native(build_c.build())
+    native = build_c.is_native(build_c.runtime_library())
     return CPU_IMPL % (" -march=native, built on this box" if native else ", portable build (no gcc on this box)")
 
 
 def cpu_solve(workload, grid, maxit, max_iterations=None, threads=None):
-    """One CPU PARSDMM run of `workload` on `grid`.  Returns (x, log, seconds of the iteration phases, seconds of
-    set-up + PARSDMM_initialize).  The operator set-up is cached between calls (it is outside the PARSDMM call in the
+    """One CPU PARSDMM run of `workload` on `grid`.  Returns ((x, log, l, y), seconds of the iteration phases, seconds
+    of set-up + PARSDMM_initialize).  The operator set-up is cached between calls (it is outside the PARSDMM call in the
     reference too)."""
     import problems as pr
     orc = pr.OracleAPI()
@@ -185,16 +223,17 @@ def cpu_solve(workload, grid, maxit, max_iterations=None, threads=None):
             cb.use_all_cores()
         else:
             cb.lib().sipref_set_threads(int(threads))
-        x, log, _, _ = cb.PARSDMM(spec["m"].copy(), ob["AtA"], ob["TD_OP"], ob["set_Prop"], ob["P_sub"], ob["cg"], opt,
-                                  constraint=ob["cons"], max_iterations=max_iterations)
+        res = cb.PARSDMM(spec["m"].copy(), ob["AtA"], ob["TD_OP"], ob["set_Prop"], ob["P_sub"], ob["cg"], opt,
+                         constraint=ob["cons"], max_iterations=max_iterations)
         if threads is not None:
             cb.use_all_cores()
     else:
         if max_iterations:
             opt.maxit = min(opt.maxit, int(max_iterations))
-        x, log, _, _ = orc.PARSDMM(spec["m"].copy(), ob["AtA"], ob["TD_OP"], ob["set_Prop"], ob["P_sub"], ob["cg"], opt)
+        res = orc.PARSDMM(spec["m"].copy(), ob["AtA"], ob["TD_OP"], ob["set_Prop"], ob["P_sub"], ob["cg"], opt)
+    log = res[1]
     t_iter = sum(v for k, v in log.timing.items() if k != "initialization")
-    return x, log, t_iter, t_setup + log.timing.get("initialization", 0.0)
+    return res, t_iter, t_setup + log.timing.get("initialization", 0.0)
 
 
 def cpu_sample_main(args):
@@ -206,11 +245,11 @@ def cpu_sample_main(args):
     sub = (n, n, max(n // f, 8))
     f_eff = n / sub[2]
     iters = args.cpu_iters
-    _, log, t_iter, t_setup = cpu_solve(args.workload, sub, 200, max_iterations=iters)
-    done = len(log.obj)
+    res, t_iter, t_setup = cpu_solve(args.workload, sub, 200, max_iterations=iters)
+    done = len(res[1].obj)
     rate_sub = done / t_iter
     return {"value": rate_sub / f_eff, "measured_on_sample": rate_sub, "iterations": done, "t_iter": t_iter, "t_setup": t_setup,
-            "sample_grid": list(sub), "factor": f_eff}
+            "sample_grid": list(sub), "factor": f_eff, "result": res}
 
 
 def run_reference(args, rank, world):
@@ -253,6 +292,8 @@ def run_reference(args, rank, world):
         "e2e": {"value": value, "unit": "iterations/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, output_arrays(last["result"]))
     print(json.dumps(line))
 
 
@@ -305,19 +346,22 @@ class DeviceProblem:
 
 
 def timed(fn, steps, barrier):
-    """K calls of fn bracketed by barrier + synchronize; returns (wall s, summed device s, iterations, launches, h2d, d2h)."""
+    """K calls of fn bracketed by barrier + synchronize; returns (wall s, summed device s, iterations, launches, h2d, d2h,
+    return value of the last call)."""
     barrier()
     t0 = time.perf_counter()
     dev_s, its, launches, h2d, d2h = 0.0, 0, 0, 0, 0
+    res = None
     for _ in range(steps):
-        _, lg, _, _ = fn()
+        res = fn()
+        lg = res[1]
         dev_s += lg.timing["device_seconds"]
         its += len(lg.obj)
         launches += lg.timing["total_launches"]
         h2d += lg.timing["h2d_bytes"]
         d2h += lg.timing["d2h_bytes"]
     barrier()
-    return time.perf_counter() - t0, dev_s, its, launches, h2d, d2h
+    return time.perf_counter() - t0, dev_s, its, launches, h2d, d2h, res
 
 
 def run_device(args, rank, world, local_rank):
@@ -367,14 +411,17 @@ def run_device(args, rank, world, local_rank):
         prob.solve(resident_io=True)
     sampler = ClockSampler(local_rank)
     sampler.start()
-    wall_res, dev_s, its, launches, _, _ = timed(lambda: prob.solve(resident_io=True), args.steps, barrier)
-    # end to end through the public API, pinned host buffers; the reference's return tuple includes l and y
-    e_steps = args.steps if args.e2e_steps <= 0 else min(args.steps, args.e2e_steps)
-    prob.solve_e2e(True)
-    wall_e2e, _, e2e_its, _, h2d, d2h = timed(lambda: prob.solve_e2e(True), e_steps, barrier)
-    prob.solve_e2e(False)
-    wall_x, _, x_its, _, h2d_x, d2h_x = timed(lambda: prob.solve_e2e(False), e_steps, barrier)
-    clocks = sampler.stop()
+    try:
+        wall_res, dev_s, its, launches, _, _, _ = timed(lambda: prob.solve(resident_io=True), args.steps, barrier)
+        # end to end through the public API, pinned host buffers; the reference's return tuple includes l and y
+        e_steps = args.steps if args.e2e_steps <= 0 else min(args.steps, args.e2e_steps)
+        prob.solve_e2e(True)
+        wall_e2e, _, e2e_its, _, h2d, d2h, e2e_last = timed(lambda: prob.solve_e2e(True), e_steps, barrier)
+        dump = output_arrays(e2e_last) if args.dump_outputs else None       # before the next leg reuses x's buffer
+        prob.solve_e2e(False)
+        wall_x, _, x_its, _, h2d_x, d2h_x, _ = timed(lambda: prob.solve_e2e(False), e_steps, barrier)
+    finally:
+        clocks = sampler.stop()
     dev_s_max, wall_e2e_max, wall_x_max, wall_res_max = reduce_max([dev_s, wall_e2e, wall_x, wall_res])
 
     # ---- roofline of the dominant kernel class from one profiled solve (CUDA events around every launch) -------
@@ -435,7 +482,7 @@ def run_device(args, rank, world, local_rank):
             xs, ls, _, _ = pp_.solve()
             xg = gather_x(pp_, xs)
             if rank == 0:
-                xo, lo, _, _ = cpu_solve(args.workload, pg, pmaxit)
+                (xo, lo, _, _), _, _ = cpu_solve(args.workload, pg, pmaxit)
                 parity[args.workload + "_reduced"] = {
                     "grid": list(pg), "maxit": pmaxit, "rel_l2": relerr(xg, xo), "iters_equal": len(ls.obj) == len(lo.obj),
                     "cg_it_equal": bool(np.array_equal(ls.cg_it, lo.cg_it)), "iterations": len(ls.obj),
@@ -453,20 +500,21 @@ def run_device(args, rank, world, local_rank):
             p2 = DeviceProblem(sip, "config2", g2)
             for _ in range(2):
                 p2.solve(resident_io=True)
-            w2, d2, it2, la2, _, _ = timed(lambda: p2.solve(resident_io=True), 5, barrier)
+            w2, d2, it2, la2, _, _, _ = timed(lambda: p2.solve(resident_io=True), args.steps, barrier)
             p2.solve_e2e(True)
-            we2, _, ite2, _, h2, dd2 = timed(lambda: p2.solve_e2e(True), 5, barrier)
+            we2, _, ite2, _, h2, dd2, _ = timed(lambda: p2.solve_e2e(True), args.steps, barrier)
             d2m, we2m = reduce_max([d2, we2])
             xs, ls, _, _ = p2.solve()
             xg = gather_x(p2, xs)
             if rank == 0:
-                c2 = {"workload": WORKLOADS["config2"] % g2, "grid": list(g2), "steps": 5, "value": it2 / d2m,
-                      "unit": "iterations/s", "ms_per_step": 1e3 * d2m / 5, "parsdmm_iterations_per_step": len(ls.obj),
-                      "e2e": {"value": ite2 / we2m, "unit": "iterations/s", "ms_per_step": 1e3 * we2m / 5,
-                              "h2d_bytes_per_step": h2 // 5, "d2h_bytes_per_step": dd2 // 5, "returns": "x, l, y, log"},
-                      "gpu_launches_per_step": la2 // 5}
+                k2 = args.steps
+                c2 = {"workload": WORKLOADS["config2"] % g2, "grid": list(g2), "steps": k2, "value": it2 / d2m,
+                      "unit": "iterations/s", "ms_per_step": 1e3 * d2m / k2, "parsdmm_iterations_per_step": len(ls.obj),
+                      "e2e": {"value": ite2 / we2m, "unit": "iterations/s", "ms_per_step": 1e3 * we2m / k2,
+                              "h2d_bytes_per_step": h2 // k2, "d2h_bytes_per_step": dd2 // k2, "returns": "x, l, y, log"},
+                      "gpu_launches_per_step": la2 // k2}
                 if not args.no_cpu:
-                    xo, lo, t_iter, t_setup = cpu_solve("config2", g2, 200)
+                    (xo, lo, _, _), t_iter, t_setup = cpu_solve("config2", g2, 200)
                     c2["parity"] = {"grid": list(g2), "rel_l2": relerr(xg, xo), "iters_equal": len(ls.obj) == len(lo.obj),
                                     "cg_it_equal": bool(np.array_equal(ls.cg_it, lo.cg_it)), "iterations": len(ls.obj),
                                     "oracle_iterations": len(lo.obj)}
@@ -475,7 +523,7 @@ def run_device(args, rank, world, local_rank):
                                                     "phases; %.1f s of set-up and initialization excluded); %s"
                                                     % (len(lo.obj), t_iter, t_setup, cpu_impl())}
                     if world == 1 and cpu_threaded_available():
-                        _, l4, t4, _ = cpu_solve("config2", g2, 200, max_iterations=8, threads=4)
+                        (_, l4, _, _), t4, _ = cpu_solve("config2", g2, 200, max_iterations=8, threads=4)
                         c2["cpu_baseline"]["threads4"] = {"value": len(l4.obj) / t4, "unit": "iterations/s", "cores": 4,
                                                           "sample": "first %d iterations (JULIA_NUM_THREADS=4 of "
                                                                     "examples/test_scaling_3D.jl:3-4)" % len(l4.obj)}
@@ -541,6 +589,8 @@ def run_device(args, rank, world, local_rank):
         "resident_wall_ms_per_step": 1e3 * wall_res_max / args.steps,
         "bench_wall_s": round(time.perf_counter() - t_wall0, 1),
     }
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
@@ -565,12 +615,18 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip every CPU leg (cpu_baseline, oracle parity)")
     ap.add_argument("--no-config2", action="store_true", help="skip the configs[1] block")
     ap.add_argument("--scaling", default="strong", choices=["strong"], help="N>1 keeps the grid fixed")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.n <= 0:
         args.n = 512 if args.workload == "config3" else 200
     if args.no_cpu:
         args.parity_size = 0
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
+    if args.dump_outputs and args.impl == "device" and world > 1:
+        ap.error("--dump-outputs needs a single process on the device arm (x, l and y stay in per-rank slabs)")
     if args.impl == "reference":
         run_reference(args, rank, world)
     else:

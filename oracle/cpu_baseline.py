@@ -31,7 +31,7 @@ _i64p, _i32p, _dp, _vp = C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C
 def lib():
     global _LIB
     if _LIB is None:
-        _LIB = C.CDLL(build_c.build())
+        _LIB = C.CDLL(build_c.runtime_library())
         _LIB.sipref_threads.restype = C.c_int
         _LIB.sipref_set_threads.restype, _LIB.sipref_set_threads.argtypes = None, [C.c_int]
         for sfx, real in (("f32", C.c_float), ("f64", C.c_double)):

@@ -1,10 +1,13 @@
 """bench.py's reference arm runs without a GPU: check its JSON line against the contract (one line, the device arm's
-metric / unit / config keys, `impl`, `cpu_baseline`, `e2e`) on a tiny grid, and that the device arm refuses to run
-without a CUDA device instead of falling back to the CPU."""
+metric / unit / config keys, `impl`, `cpu_baseline`, `e2e`) on a tiny grid, its --dump-outputs files, that a run
+writes nothing into the tree, and that the device arm refuses to run without a CUDA device instead of falling back to
+the CPU."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,6 +33,37 @@ def test_reference_arm_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and "sub-volume" in cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": "iterations/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def _tree_state():
+    """(path, size, mtime) of every file where a run could leave bytecode or a build of the CPU baseline."""
+    out = set()
+    for top in ("__pycache__", "oracle", "setintersectionprojection.jl_b200", "tests"):
+        for dirpath, _, files in os.walk(os.path.join(ROOT, top)):
+            for f in files:
+                st = os.stat(os.path.join(dirpath, f))
+                out.add((os.path.join(dirpath, f), st.st_size, st.st_mtime_ns))
+    return out
+
+
+def test_reference_arm_dump_outputs(tmp_path):
+    """--dump-outputs: x, l_<i>, y_<i> and the log's arrays of the last step as finite float32 / float64 .npy files, the
+    same on a second run with the same arguments; neither run writes into the tree."""
+    before = _tree_state()
+    outs = []
+    for run in ("a", "b"):
+        r = _run("--impl", "reference", "--size", "32", "--cpu-sub", "2", "--steps", "1", "--warmup", "0",
+                 "--dump-outputs", str(tmp_path / run), env={"PYTHONDONTWRITEBYTECODE": ""})
+        assert r.returncode == 0, r.stderr[-2000:]
+        outs.append({p.stem: np.load(p) for p in (tmp_path / run).glob("*.npy")})
+    assert _tree_state() == before
+    a, b = outs
+    assert {"x", "l_0", "y_0", "log_obj", "log_rho", "log_cg_it"} <= set(a) and set(a) == set(b)
+    assert a["x"].shape == (32 * 32 * 16,) and a["log_evol_x"].shape == (a["log_obj"].size - 1,)
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64), k
+        assert np.all(np.isfinite(a[k])), k
+        assert np.allclose(a[k], b[k], rtol=1e-5, atol=0), k
 
 
 def test_reference_arm_other_ranks_exit_silently():
