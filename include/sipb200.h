@@ -239,7 +239,11 @@ int sipb_problem_destroy(sipb_problem* pb);
  * fine problem's device buffers.  Replaces the Interpolations.jl calls of PARSDMM_multi_level.jl:61-67 and
  * interpolate_y_l.jl:32-91.  Each segment resamples one column-major box: `vec` = -1 for x, or the set index
  * for l and y (both are resampled); offsets are element offsets inside that vector; the sampling positions
- * are range(1, stop=n_src, length=n_dst) per axis with half-way positions rounded up. */
+ * are range(1, stop=n_src, length=n_dst) per axis with half-way positions rounded up.
+ * Slab-decomposed problems (both levels on the same communicator): the segments are global — offsets and shapes
+ * address the whole vector in the reference's row-block-major order — and the call is collective: every rank passes
+ * the same segments, the coarse vectors are gathered whole on every rank (ncclSend / ncclRecv), and each rank
+ * receives its own planes of the fine x, l, y.  Both problems must be slab-decomposed, or neither. */
 typedef struct sipb_resample_seg {
   int32_t vec;
   int32_t reserved;

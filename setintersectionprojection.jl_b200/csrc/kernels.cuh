@@ -1662,19 +1662,20 @@ __device__ __forceinline__ void spec_hist_add(SpecCtx& sc, T v) {
 }
 
 // nearest-neighbour resampling of a column-major box (multilevel warm starts): sample k of an axis reads source
-// index floor(pos + 1/2) - 1 with pos = 1 + k (ns-1)/(nd-1), evaluated in exact integer arithmetic
+// index floor(pos + 1/2) - 1 with pos = 1 + k (ns-1)/(nd-1), evaluated in exact integer arithmetic.
+// Only the destination elements [q0, q1) of the box are written, to dst[0 .. q1-q0) (slabs: the rows a rank stores);
+// the source is the whole box.
 __device__ __forceinline__ long long nn_src_index(long long k, long long ns, long long nd) {
   if (nd <= 1) return 0;
   return (3 * (nd - 1) + 2 * k * (ns - 1)) / (2 * (nd - 1)) - 1;
 }
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_resample_nn(const T* __restrict__ src, T* __restrict__ dst, i64 ns0,
-                                                          i64 ns1, i64 ns2, i64 nd0, i64 nd1, i64 nd2) {
-  const i64 total = nd0 * nd1 * nd2;
-  for (i64 q = (i64)blockIdx.x * blockDim.x + threadIdx.x; q < total; q += (i64)gridDim.x * blockDim.x) {
+                                                          i64 ns1, i64 ns2, i64 nd0, i64 nd1, i64 nd2, i64 q0, i64 q1) {
+  for (i64 q = q0 + (i64)blockIdx.x * blockDim.x + threadIdx.x; q < q1; q += (i64)gridDim.x * blockDim.x) {
     const i64 i = q % nd0, t = q / nd0, j = t % nd1, kk = t / nd1;
     const i64 si = nn_src_index(i, ns0, nd0), sj = nn_src_index(j, ns1, nd1), sk = nn_src_index(kk, ns2, nd2);
-    dst[q] = src[si + ns0 * (sj + ns1 * sk)];
+    dst[q - q0] = src[si + ns0 * (sj + ns1 * sk)];
   }
 }
 

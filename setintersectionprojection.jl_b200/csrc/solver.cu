@@ -1537,14 +1537,76 @@ struct Problem : sipb_problem {
     return SIPB_OK;
   }
 
-  // device-side nearest-neighbour warm start from a coarser problem (PARSDMM_multi_level.jl:61-82)
+  // Row blocks of a vector in the global (row-block major) order on slabs: first global row, rows per z plane,
+  // and whether the block differences along z (a D_z block has one row plane fewer than the grid).
+  struct SlabBlock { i64 start, plane; bool dz; };
+  std::vector<SlabBlock> slab_blocks(int vec) const {
+    std::vector<SlabBlock> out;
+    if (vec < 0 || sets[vec]->op.kind == SIPB_OP_IDENTITY) {
+      out.push_back({0, n[0] * n[1], false});
+      return out;
+    }
+    const OpDev& op = sets[vec]->op;
+    i64 start = 0;
+    for (int b = 0; b < op.nblk; ++b) {
+      const int a = op.axis[b];
+      const SlabBlock k{start, (n[0] - (a == 0)) * (n[1] - (a == 1)), a == 2};
+      out.push_back(k);
+      start += k.plane * (n[2] - k.dz);
+    }
+    return out;
+  }
+  // planes [k0, k1) of block `k` stored by `rank` (the rule of SlabGeom::nz_rows)
+  std::pair<i64, i64> slab_planes(const SlabBlock& k, int rank) const {
+    const i64 nz = n[2], k0 = nz * rank / ctx->world, k1 = nz * (rank + 1) / ctx->world;
+    return {k0, k.dz ? std::min(k1, nz - 1) : k1};
+  }
+  // Collective: every rank's rows of the slab vector `local` (vector id `vec`: -1 = x, else a set's l / y) land at
+  // their global positions in `glob`, so each rank holds the whole vector in the reference's order.
+  int gather_global(int vec, const T* local, T* glob) {
+    sipb_ctx* c = ctx;
+    const auto blks = slab_blocks(vec);
+    i64 loc = 0;
+    for (const auto& k : blks) {          // own rows: a device copy
+      const auto pl = slab_planes(k, c->rank);
+      const i64 cnt = k.plane * (pl.second - pl.first);
+      if (cnt > 0)
+        SIPB_CUDA_CHECK(cudaMemcpyAsync(glob + k.start + k.plane * pl.first, local + loc, cnt * sizeof(T),
+                                        cudaMemcpyDeviceToDevice, c->stream));
+      loc += cnt;
+    }
+    c->nccl_calls++;
+    SIPB_NCCL_CHECK(NCCL(GroupStart)());
+    loc = 0;
+    for (const auto& k : blks) {
+      const auto mine = slab_planes(k, c->rank);
+      const i64 cnt = k.plane * (mine.second - mine.first);
+      for (int r = 0; r < c->world; ++r) {
+        if (r == c->rank) continue;
+        const auto pl = slab_planes(k, r);
+        const i64 rcnt = k.plane * (pl.second - pl.first);
+        if (cnt > 0) SIPB_NCCL_CHECK(NCCL(Send)(local + loc, (size_t)cnt, nccl_type(), r, c->comm, c->stream));
+        if (rcnt > 0)
+          SIPB_NCCL_CHECK(NCCL(Recv)(glob + k.start + k.plane * pl.first, (size_t)rcnt, nccl_type(), r, c->comm, c->stream));
+      }
+      loc += cnt;
+    }
+    SIPB_NCCL_CHECK(NCCL(GroupEnd)());
+    return SIPB_OK;
+  }
+
+  // device-side nearest-neighbour warm start from a coarser problem (PARSDMM_multi_level.jl:61-82).  On slabs the
+  // segments address global vectors: each coarse vector is gathered whole on every rank, and every rank resamples the
+  // rows it stores of each fine vector.
   int warm_from(sipb_problem* coarse_, const sipb_resample_seg* segs, int nseg) override {
     SIPB_REQUIRE(finalized && coarse_ && segs, SIPB_E_STATE, "warm_from needs two finalized problems");
     SIPB_REQUIRE(coarse_->dtype == dtype && coarse_->ctx == ctx, SIPB_E_INVALID, "problems differ in dtype / context");
-    SIPB_REQUIRE(!sg.on, SIPB_E_UNSUPPORTED, "device warm starts are single-GPU (multilevel levels are small)");
     Problem<T>* co = static_cast<Problem<T>*>(coarse_);
     SIPB_REQUIRE(co->finalized && co->sets.size() == sets.size(), SIPB_E_INVALID, "level problems have different sets");
+    SIPB_REQUIRE(co->sg.on == sg.on, SIPB_E_INVALID, "one level problem is slab-decomposed, the other is not");
     sipb_ctx* c = ctx;
+    const int p = (int)sets.size();
+    // validate every segment before the first collective, so that all ranks fail alike
     for (int q = 0; q < nseg; ++q) {
       const sipb_resample_seg& g = segs[q];
       i64 ns = 1, nd = 1;
@@ -1553,23 +1615,53 @@ struct Problem : sipb_problem {
         ns *= g.src_shape[a];
         nd *= g.dst_shape[a];
       }
-      const T* srcs[2];
-      T* dsts[2];
-      int nv = 0;
-      i64 src_len, dst_len;
-      if (g.vec < 0) {
-        srcs[0] = co->x.p; dsts[0] = x.p; nv = 1; src_len = co->N; dst_len = N;
-      } else {
-        SIPB_REQUIRE(g.vec < (int)sets.size(), SIPB_E_INVALID, "set index out of range");
-        srcs[0] = co->sets[g.vec]->l.p; dsts[0] = sets[g.vec]->l.p;
-        srcs[1] = co->sets[g.vec]->y.p; dsts[1] = sets[g.vec]->y.p;
-        nv = 2; src_len = co->sets[g.vec]->M; dst_len = sets[g.vec]->M;
-      }
+      SIPB_REQUIRE(g.vec >= -1 && g.vec < p, SIPB_E_INVALID, "set index out of range");
+      const i64 src_len = g.vec < 0 ? (sg.on ? co->Nglob : co->N) : (sg.on ? co->sets[g.vec]->Mglob : co->sets[g.vec]->M);
+      const i64 dst_len = g.vec < 0 ? (sg.on ? Nglob : N) : (sg.on ? sets[g.vec]->Mglob : sets[g.vec]->M);
       SIPB_REQUIRE(g.src_off >= 0 && g.src_off + ns <= src_len && g.dst_off >= 0 && g.dst_off + nd <= dst_len,
                    SIPB_E_INVALID, "resampling segment outside its vector");
-      for (int v = 0; v < nv; ++v)
-        LAUNCH(c, KC_OP_APPLY, k_resample_nn<T>, c->grid_for(nd), srcs[v] + g.src_off, dsts[v] + g.dst_off, g.src_shape[0],
-               g.src_shape[1], g.src_shape[2], g.dst_shape[0], g.dst_shape[1], g.dst_shape[2]);
+    }
+    DevBuf<T> stage;       // slabs: one whole coarse vector at a time
+    if (sg.on) {
+      i64 big = co->Nglob;
+      for (auto& S : co->sets) big = std::max<i64>(big, S->Mglob);
+      SIPB_CUDA_CHECK(stage.alloc((size_t)big));
+    }
+    // source vectors in the order x, l_0, y_0, l_1, y_1, ...
+    for (int v = -1; v < 2 * p; ++v) {
+      const int vec = v < 0 ? -1 : v / 2;
+      T* dst_vec = vec < 0 ? x.p : (v % 2 ? sets[vec]->y.p : sets[vec]->l.p);
+      const T* src_vec = vec < 0 ? co->x.p : (v % 2 ? co->sets[vec]->y.p : co->sets[vec]->l.p);
+      bool used = false;
+      for (int q = 0; q < nseg; ++q) used = used || segs[q].vec == vec;
+      if (!used) continue;        // every rank passes the same segments, so all ranks skip the same gathers
+      if (sg.on) {
+        int rc = co->gather_global(vec, src_vec, stage.p);
+        if (rc) return rc;
+        src_vec = stage.p;
+      }
+      for (int q = 0; q < nseg; ++q) {
+        const sipb_resample_seg& g = segs[q];
+        if (g.vec != vec) continue;
+        const i64 nd = g.dst_shape[0] * g.dst_shape[1] * g.dst_shape[2];
+        auto launch = [&](T* dst, i64 q0, i64 q1) {
+          LAUNCH(c, KC_OP_APPLY, k_resample_nn<T>, c->grid_for(q1 - q0), src_vec + g.src_off, dst, g.src_shape[0],
+                 g.src_shape[1], g.src_shape[2], g.dst_shape[0], g.dst_shape[1], g.dst_shape[2], q0, q1);
+        };
+        if (!sg.on) {
+          launch(dst_vec + g.dst_off, 0, nd);
+          continue;
+        }
+        // this rank's rows of each destination block: one global range per block, stored contiguously
+        i64 loc = 0;
+        for (const auto& k : slab_blocks(vec)) {
+          const auto pl = slab_planes(k, c->rank);
+          const i64 gs = k.start + k.plane * pl.first, ge = k.start + k.plane * pl.second;
+          const i64 a = std::max(gs, (i64)g.dst_off), b = std::min(ge, (i64)g.dst_off + nd);
+          if (a < b) launch(dst_vec + loc + (a - gs), a - g.dst_off, b - g.dst_off);
+          loc += ge - gs;
+        }
+      }
     }
     SIPB_CUDA_CHECK(cudaGetLastError());
     SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));

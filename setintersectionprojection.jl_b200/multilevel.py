@@ -12,6 +12,7 @@ index tables are built in exact integer arithmetic.
 from __future__ import annotations
 
 import copy
+import time
 
 import numpy as np
 
@@ -67,17 +68,25 @@ def setup_multi_level_PARSDMM(m, n_levels, coarsening_factor, comp_grid, constra
     """-> (TD_OP_levels, AtA_levels, P_sub_levels, set_Prop_levels, comp_grid_levels, constraint_level)
     (setup_multi_level_PARSDMM.jl:7-14,135)."""
     TF = m.dtype.type
+    grids = [comp_grid]
+    for lev in range(1, n_levels):
+        n = tuple(int(np.round(v / coarsening_factor ** lev)) for v in comp_grid.n)           # :66
+        d = tuple((vn / nn) * vd for vn, nn, vd in zip(comp_grid.n, n, comp_grid.d))          # :82
+        grids.append(compgrid(d, n))
+    if dd.active() and len(comp_grid.n) == 3:
+        for lev, grid in enumerate(grids):
+            if int(grid.n[2]) < dd.world():
+                raise ValueError("level %d (grid %s) has %d z planes, fewer than the %d ranks of the slab decomposition; "
+                                 "use fewer levels or fewer ranks" % (lev, tuple(int(v) for v in grid.n), int(grid.n[2]),
+                                                                      dd.world()))
     out = ([], [], [], [], [])
     level_constraint = None
-    for lev in range(n_levels):
+    for lev, grid in enumerate(grids):
         if lev == 0:
-            grid, cons = comp_grid, constraint
+            cons = constraint
         else:
             if level_constraint is None:
                 level_constraint = copy.deepcopy(constraint)             # :61 (after the fine-level TF cast)
-            n = tuple(int(np.round(v / coarsening_factor ** lev)) for v in comp_grid.n)       # :66
-            d = tuple((vn / nn) * vd for vn, nn, vd in zip(comp_grid.n, n, comp_grid.d))      # :82
-            grid = compgrid(d, n)
             cons = level_constraint = constraint2coarse(level_constraint, grid, coarsening_factor)   # :87
         P_sub, TD_OP, set_Prop = setup_constraints(cons, grid, TF)
         TD_OP, AtA, _, _ = PARSDMM_precompute_distribute(TD_OP, set_Prop, grid, options)
@@ -142,6 +151,18 @@ def warm_start_segments(set_Prop_levels, comp_grid_levels, dim3, i):
     return segs
 
 
+def _host_warm_start(x, l, y, TD_OP_coarse, set_Prop_levels, comp_grid_levels, dim3, i):
+    """x, l, y of level i+1 resampled on the host to level i (global vectors).  On slabs `l`, `y` are this rank's
+    slabs: they are gathered into the reference's global order first (`x` is already global); PARSDMM scatters the
+    global result again."""
+    if dd.active():
+        l = [dd.gather_td(v, A) for v, A in zip(l, TD_OP_coarse)]
+        y = [dd.gather_td(v, A) for v, A in zip(y, TD_OP_coarse)]
+    x = resample_nn(x, comp_grid_levels[i + 1].n, comp_grid_levels[i].n)       # :61-67
+    l, y = interpolate_y_l(l, y, set_Prop_levels, comp_grid_levels, dim3, i)   # :74
+    return x, l, y
+
+
 def _device_warm_start(dev_fine, dev_coarse, segs):
     arr = (_lib.ResampleSeg * len(segs))()
     for q, (vec, so, do, ss, ds) in enumerate(segs):
@@ -155,36 +176,47 @@ def PARSDMM_multi_level(m, TD_OP_levels, AtA_levels, P_sub_levels, set_Prop_leve
                         x_ini=None, l_ini=None, y_ini=None, *, device_resample=True):
     """-> (x, log_PARSDMM, l, y) on the finest grid (PARSDMM_multi_level.jl:8-19,88).
 
-    With `device_resample` (default, single GPU) x, l, y never leave the GPU between levels: a resampling
-    kernel writes the warm start straight into the finer problem's device buffers; only the finest level's
-    x, l, y are copied back.  Otherwise the host-side `resample_nn` / `interpolate_y_l` are used."""
+    With `device_resample` (default) x, l, y never leave the GPU between levels: a resampling kernel writes the
+    warm start straight into the finer problem's device buffers; only the finest level's x, l, y are copied back.
+    Otherwise the host-side `resample_nn` / `interpolate_y_l` are used.
+
+    Multi-GPU slabs (after `distributed.init`, 3-D problems): every level is slab-decomposed along z.  On the device
+    path each transition gathers the coarse x, l, y on every rank (ncclSend / ncclRecv) and each rank resamples its
+    own planes; the host path gathers l, y with `distributed.gather_td`.  As for `PARSDMM`, the returned x is global
+    and l, y are this rank's slabs.
+
+    `log.timing["transition_seconds"]` holds the host time of each level-to-level warm start, coarsest first."""
     TF = m.dtype.type
     n_levels = len(TD_OP_levels)
     rho_orig = copy.deepcopy(options.rho_ini)
     fine = tuple(comp_grid_levels[0].n)
     dim3 = len(fine) == 3 and fine[2] > 1
     m_levels = [m] + [resample_nn(m, fine, comp_grid_levels[k].n) for k in range(1, n_levels)]
-    logs = []
+    logs, transitions = [], []
     x, l, y = x_ini, l_ini, y_ini
-    on_device = bool(device_resample) and not dd.active() and not options.Minkowski
+    on_device = bool(device_resample) and not options.Minkowski
     try:
         for k in range(n_levels - 1, -1, -1):
             kw = {}
+            t0 = time.perf_counter()
             if k == n_levels - 1:
                 options.zero_ini_guess = True                                    # coarsest level: zero guess (:53)
             elif on_device:
                 devs = [device_problem(m.dtype, AtA_levels[q], TD_OP_levels[q], set_Prop_levels[q], P_sub_levels[q],
                                        comp_grid_levels[q], options) for q in (k, k + 1)]
+                t0 = time.perf_counter()
                 _device_warm_start(devs[0], devs[1], warm_start_segments(set_Prop_levels, comp_grid_levels, dim3, k))
                 options.zero_ini_guess = False                                   # :81
                 x, l, y = None, None, None
                 kw = dict(warm_resident=True)
             else:
-                x = resample_nn(x, comp_grid_levels[k + 1].n, comp_grid_levels[k].n)       # :61-67
-                l, y = interpolate_y_l(l, y, set_Prop_levels, comp_grid_levels, dim3, k)   # :74
+                x, l, y = _host_warm_start(x, l, y, TD_OP_levels[k + 1], set_Prop_levels, comp_grid_levels, dim3, k)
                 options.zero_ini_guess = False                                   # :81
+            if k < n_levels - 1:
+                transitions.append(time.perf_counter() - t0)
             if on_device and k > 0:
                 kw["return_ly"] = False                                          # l, y stay on the device
+                kw["gather_result"] = False                                      # slabs: x too
             x, log, l, y = PARSDMM(m_levels[k], AtA_levels[k], TD_OP_levels[k], set_Prop_levels[k], P_sub_levels[k],
                                    comp_grid_levels[k], options, x, l, y, **kw)
             options.rho_ini = [TF(v) for v in log.rho[-1, :]]                    # :57 / :83
@@ -193,4 +225,5 @@ def PARSDMM_multi_level(m, TD_OP_levels, AtA_levels, P_sub_levels, set_Prop_leve
         options.rho_ini = rho_orig                                               # :87
     log.timing["levels"] = [lg.timing for lg in logs]
     log.timing["level_iterations"] = [len(lg.obj) for lg in logs]
+    log.timing["transition_seconds"] = transitions
     return x, log, l, y
