@@ -303,6 +303,27 @@ int sipb_bench_spmv2(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, int w
  * otherwise the generic kernel.  Unit-test entry point of the tiled SpMV. */
 int sipb_cds_spmv_grid(sipb_ctx* ctx, int dtype, const int64_t* n, int nd, const void* R, const int64_t* offsets,
                        const void* x, void* y, int* used_tiled);
+/* The SpMV of the CG exactly as the solver launches it, on a 3-D grid n with Q given either as a stencil-class table
+ * `tab` (host TF[27][nd], row cls = (c(k)*3 + c(j))*3 + c(i) as in sipb_problem_set_ata_classes; R = NULL) or as CDS
+ * arrays `R` (column-major [N x nd]; tab = NULL).  mode 1: y = Q*x (cg.jl:85, CDS_MVp_MT.jl:9-25) and sums[0] =
+ * dot(x, y) (cg.jl:88); mode 2, the CG prologue (argmin_x.jl:33-37, cg.jl:47-61): r = b - Q*x, p = r, x_old = x,
+ * sums[0] = dot(b,b), sums[1] = dot(r,r).  tiled = 1: the TMA-staged plane sweep of spmv_tile.cuh (SIPB_E_UNSUPPORTED
+ * when the planner rejects the grid; mode 2 has a class-form body only), 0: the generic grid-stride kernels.
+ * geom (optional) receives the plan: {ok, TJ, JT, KC, NS, grid, gpl, LPP}.  Unit-test entry point. */
+int sipb_tile_probe(sipb_ctx* ctx, int dtype, const int64_t* n, int nd, const int64_t* offsets, const void* tab,
+                    const void* R, const void* x, const void* b, int mode, int tiled, void* y, void* r, void* p,
+                    void* x_old, double* sums, int* geom);
+/* The single-GPU cardinality projection (project_cardinality!.jl:3-21) as the PARSDMM loop runs it: v (M entries) is
+ * the input of the y/l update of a one-set problem with the identity operator, l = 0 and rho = gamma = 1 (so pass 1
+ * produces s = 0 + v: v itself, except that a -0.0 becomes +0.0 as in the reference's A*x), and `guess`
+ * is the previous threshold key the speculative levels are built around.  path 0 / 1: pass 1 without / with the
+ * speculative select levels, the search, the tie counts and pass 2 zeroing the ties beyond the quota (deferred tie
+ * handling); path 2: the sipb_project sequence (ties zeroed in place).  y receives the projection; stats (optional,
+ * int64[8]) = {threshold magnitude key, tie quota, keys equal to the threshold, ties to resolve (0/1), histogram passes
+ * that ran, per-chunk tie table valid (0/1), chunk length of the tie kernels, chunk settled in place (-1: none)}.
+ * Unit-test entry point. */
+int sipb_select_probe(sipb_ctx* ctx, int dtype, int64_t M, const void* v, int64_t k, uint64_t guess, int path, void* y,
+                      int64_t* stats);
 
 #ifdef __cplusplus
 }

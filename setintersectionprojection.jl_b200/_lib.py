@@ -115,6 +115,8 @@ SYMBOLS = [
     ("sipb_bench_spmv", _I, [_VP, _I, _I, _PI64, _I, _I, _I, _PD, _PI64]),
     ("sipb_bench_spmv2", _I, [_VP, _I, _I, _PI64, _I, _I, _I, _I, _I, _PD, _PI64]),
     ("sipb_cds_spmv_grid", _I, [_VP, _I, _PI64, _I, _VP, _PI64, _VP, _VP, _PI]),
+    ("sipb_tile_probe", _I, [_VP, _I, _PI64, _I, _PI64, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP, _VP, _VP, _PD, _PI]),
+    ("sipb_select_probe", _I, [_VP, _I, _I64, _VP, _I64, C.c_uint64, _I, _VP, _PI64]),
 ]
 
 _lib = None

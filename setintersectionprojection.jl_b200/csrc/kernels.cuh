@@ -1508,6 +1508,8 @@ struct SelState {
   int key_bits;
   int dbits;                      // digit width of this search
   int table_valid;                // the last level's per-block histograms are in the tie table (single GPU)
+  int levels_run;                 // k_radix_hist launches of this search that histogrammed a level (the rest were decided
+                                  //   by the speculation and returned at once); read by the select probe
 };
 
 // Choose the digit bucket that contains the k_rem-th largest key among the current prefix bucket, from the level
@@ -1585,6 +1587,7 @@ __global__ void __launch_bounds__(kThreads) k_radix_hist(i64 M, const T* __restr
   const unsigned long long mask = (unsigned long long)(nb - 1);
   const unsigned long long prefix = st->prefix;
   const bool all_match = bl >= st->key_bits;
+  if (blockIdx.x == 0 && threadIdx.x == 0) st->levels_run += 1;
   for (int t = threadIdx.x; t < nb; t += blockDim.x) sh[t] = 0u;
   __syncthreads();
   // rows [lo, hi) of this block, visited with stride `step` after the block's / grid's first pass (chunk > 0: the block's

@@ -404,6 +404,7 @@ __global__ void __launch_bounds__(256) k_sel_begin(long long k, long long M, Sel
     st->k_rem = (unsigned long long)(k > 0 ? k : 0);
     st->count_eq = 0ull;
     st->table_valid = 0;
+    st->levels_run = 0;
     st->bits_left = (pp->keep_all || pp->keep_none) ? 0 : st->key_bits;
   }
   for (int b = threadIdx.x; b < kSelBins; b += blockDim.x) st->hist[b] = 0ull;
@@ -452,13 +453,15 @@ __global__ void __launch_bounds__(256) k_sel_begin(long long k, long long M, Sel
   __syncthreads();
   for (int b = threadIdx.x; b < (kSpecLevels - 1) * kSelBins; b += blockDim.x) st->spec[b] = 0ull;
 }
+// need_ties also when the threshold magnitude is 0 (k > nnz): the surplus zeros then become +0.0, as
+// x[sort_ind[k+1:end]] .= 0 writes them (project_cardinality!.jl:19); a -0.0 inside the quota stays -0.0
 template <typename T>
 __global__ void k_sel_end(SelState* st, ProjParams<T>* pp) {
   if (pp->keep_all || pp->keep_none) return;
   pp->key_thr = st->prefix;
   pp->quota = st->k_rem;
   pp->count_eq = st->count_eq;
-  pp->need_ties = (st->count_eq > st->k_rem && st->prefix > 0ull) ? 1 : 0;
+  pp->need_ties = (st->count_eq > st->k_rem) ? 1 : 0;
 }
 
 // wrappers that read the tie parameters from device memory (no host round trip)
@@ -3297,6 +3300,170 @@ static int cds_spmv_grid_impl(sipb_ctx* c, const int64_t* n, int nd, const void*
   return SIPB_OK;
 }
 
+// The SpMV kernels of the CG as the solver launches them (unit tests): the argument block of a problem that holds Q in
+// class form (tab, uploaded like Q_tab and opted in by tile_prepare) or as CDS arrays (R), the tile geometry of
+// finalize, and the MODE 1 (y = Q x, dot(x, y)) or MODE 2 (CG prologue) kernel, tiled or generic.
+template <typename T>
+static int tile_probe_impl(sipb_ctx* c, const int64_t* n, int nd, const int64_t* offs, const void* tab, const void* R,
+                           const void* x, const void* b, int mode, int tiled, void* y, void* r, void* p, void* x_old,
+                           double* sums, int* geom) {
+  const i64 N = n[0] * n[1] * n[2];
+  const double hh[3] = {1, 1, 1};
+  Problem<T> PB(c, sizeof(T) == 4 ? SIPB_F32 : SIPB_F64, 3, n, hh, false, true);
+  PB.q_offs.assign(offs, offs + nd);
+  PB.q_classes = tab != nullptr;
+  if (PB.q_classes) {
+    SIPB_CUDA_CHECK(PB.Q_tab.alloc((size_t)kMaxClasses * nd));
+    SIPB_CUDA_CHECK(cudaMemsetAsync(PB.Q_tab.p, 0, (size_t)kMaxClasses * nd * sizeof(T), c->stream));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(PB.Q_tab.p, tab, (size_t)27 * nd * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+  } else {
+    int rc = upload_cds<T>(c, N, nd, R, PB.ld, PB.Q);
+    if (rc) return rc;
+  }
+  const TileGeom tg = plan_tile<T>(3, n, false, PB.q_offs, n[2], 0, false, false, c->num_sms);
+  if (geom) {
+    const int gv[8] = {tg.ok, tg.TJ, tg.JT, tg.KC, tg.NS, tg.grid, tg.gpl, tg.LPP};
+    memcpy(geom, gv, sizeof(gv));
+  }
+  SIPB_REQUIRE(!tiled || tg.ok, SIPB_E_UNSUPPORTED, "the tiled SpMV does not handle this grid");
+  SIPB_REQUIRE(!(tiled && mode == 2 && !PB.q_classes), SIPB_E_UNSUPPORTED, "the tiled CG prologue has a class-form body only");
+  if (tiled && PB.q_classes) { int rc = tile_prepare<T>(tg); if (rc) return rc; }
+  DevBuf<T> dx, dy, db, dr, dp, dxo;
+  SIPB_CUDA_CHECK(dx.alloc((size_t)N));
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(dx.p, x, N * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+  const i64 nvecN = (N + Vec<T>::W - 1) / Vec<T>::W;
+  if (mode == 1) {
+    SIPB_CUDA_CHECK(dy.alloc((size_t)N));
+    const SpmvArgs<T> a = PB.spmv_args(dx.p, dy.p);
+    if (tiled) {
+      const TileInit<T> ti{nullptr, nullptr, nullptr, nullptr};
+      int rc = launch_tile<T, 1>(c, KC_SPMV_DOT, tg, !PB.q_classes, a, ti, c->d_scal, nullptr, nullptr, c->cd_off);
+      if (rc) return rc;
+    } else {
+      LAUNCH(c, KC_SPMV_DOT, (k_spmv<T, true>), c->grid_fit((const void*)k_spmv<T, true>, nvecN), a, c->rs, c->d_scal,
+             (const int*)nullptr, c->cd_off);
+    }
+    SIPB_CUDA_CHECK(cudaGetLastError());
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(y, dy.p, N * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(sums, c->d_scal, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    SIPB_CUDA_CHECK(cudaMemsetAsync(c->d_scal, 0, sizeof(double), c->stream));
+  } else {
+    SIPB_CUDA_CHECK(db.alloc((size_t)N));
+    SIPB_CUDA_CHECK(dr.alloc((size_t)N));
+    SIPB_CUDA_CHECK(dp.alloc((size_t)N));
+    SIPB_CUDA_CHECK(dxo.alloc((size_t)N));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(db.p, b, N * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+    const SpmvArgs<T> a = PB.spmv_args(dx.p, nullptr);
+    if (tiled) {
+      const TileInit<T> ti{db.p, dr.p, dp.p, dxo.p};
+      int rc = launch_tile<T, 2>(c, KC_CG_INIT, tg, false, a, ti, nullptr, nullptr, c->d_cg, c->cd_off);
+      if (rc) return rc;
+    } else {
+      LAUNCH(c, KC_CG_INIT, k_cg_init<T>, c->grid_for(nvecN), a, (const T*)db.p, dr.p, dp.p, dxo.p, c->rs, c->d_cg, c->cd_off);
+    }
+    SIPB_CUDA_CHECK(cudaGetLastError());
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(r, dr.p, N * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(p, dp.p, N * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(x_old, dxo.p, N * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(sums, &c->d_cg->bb, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));   // bb, rr
+  }
+  SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));
+  return SIPB_OK;
+}
+
+// The single-GPU cardinality select (unit tests), on a one-set problem with the identity operator, l = 0 and
+// rho = gamma = 1, so that pass 1 of the y/l update produces v itself.  path 0 / 1: the sequence of the PARSDMM loop
+// with the speculative levels off / on (pass 1, projector_params with deferred ties, pass 2); path 2: the sipb_project
+// sequence (ties zeroed in place, then the apply pass).
+template <typename T>
+static int select_probe_impl(sipb_ctx* c, int64_t M, const void* v, int64_t k, uint64_t guess, int path, void* y,
+                             int64_t* stats) {
+  const int64_t nn[3] = {M, 1, 1};
+  const double hh[3] = {1, 1, 1};
+  Problem<T> P(c, sizeof(T) == 4 ? SIPB_F32 : SIPB_F64, 2, nn, hh, false, true);
+  SetT<T> S;
+  memset(&S.desc, 0, sizeof(S.desc));
+  S.desc.set_kind = SIPB_SET_CARDINALITY;
+  S.desc.op_kind = SIPB_OP_IDENTITY;
+  S.desc.k = k;
+  S.M = M;
+  S.Mglob = M;
+  S.op = identity_over(M);
+  DevBuf<T> dv;
+  SIPB_CUDA_CHECK(dv.alloc((size_t)M));
+  SIPB_CUDA_CHECK(S.y.alloc((size_t)M));
+  SIPB_CUDA_CHECK(S.l.alloc((size_t)M));
+  SIPB_CUDA_CHECK(S.y_old.alloc((size_t)M));
+  SIPB_CUDA_CHECK(S.s.alloc((size_t)M));
+  SIPB_CUDA_CHECK(S.pp_y.alloc(1));
+  SIPB_CUDA_CHECK(S.warm.alloc(2));
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(dv.p, v, M * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(S.l.p, 0, M * sizeof(T), c->stream));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(S.y_old.p, 0, M * sizeof(T), c->stream));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(S.warm.p, 0, 2 * sizeof(double), c->stream));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(S.pp_y.p, 0, sizeof(ProjParams<T>), c->stream));
+  const unsigned long long g64 = guess;
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(&S.pp_y.p->key_thr, &g64, sizeof(g64), cudaMemcpyHostToDevice, c->stream));
+  const int slot = 10;
+  i64 tie_chunk = 0;
+  if (path == 2) {
+    // project_impl: statistics, parameters with ties zeroed in place, the apply pass
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(S.y.p, dv.p, M * sizeof(T), cudaMemcpyDeviceToDevice, c->stream));
+    LAUNCH(c, KC_VEC_STATS, k_vec_stats<T>, c->grid_for(M), M, S.y.p, c->rs, c->d_scal + slot);
+    int rc = P.projector_params(S, S.y.p, slot, S.pp_y.p, S.warm.p, true);
+    if (rc) return rc;
+    LAUNCH(c, KC_FEAS, k_feas_dyn<T>, c->grid_for(M), M, S.y.p, (const T*)nullptr, P.proj_static(S, (T)1),
+           (const ProjParams<T>*)S.pp_y.p, 1, c->rs, c->d_scal);
+  } else {
+    // Problem::solve, y/l update of a vector-mode cardinality set on one GPU
+    const bool spec = path == 1;
+    YlArgs<T> ya;
+    memset(&ya, 0, sizeof(ya));
+    ya.op = S.op;
+    ya.P = P.proj_static(S, (T)1);
+    ya.x = dv.p; ya.y = S.y.p; ya.l = S.l.p; ya.y_old = S.y_old.p; ya.s = S.s.p;
+    ya.rho = (T)1; ya.gamma = (T)1;
+    const i64 nvecM = (M + Vec<T>::W - 1) / Vec<T>::W;
+    if (spec)
+      LAUNCH(c, KC_YL_PASS1, (k_yl_spec<T>), c->grid_fit((const void*)k_yl_spec<T>, nvecM), ya, c->rs, c->d_scal + slot,
+             &c->d_sel->spec_above, c->d_sel->spec, (const ProjParams<T>*)S.pp_y.p);
+    else
+      LAUNCH(c, KC_YL_PASS1, (k_yl<T, 1, false>), c->grid_fit((const void*)k_yl<T, 1, false>, nvecM), ya, c->rs,
+             c->d_scal + slot);
+    int rc = P.projector_params(S, S.y.p, slot, S.pp_y.p, S.warm.p, true, spec, &tie_chunk);
+    if (rc) return rc;
+    ya.dyn = S.pp_y.p;
+    if (tie_chunk > 0) { ya.P.tie_base = c->d_tie_base; ya.P.tie_chunk = tie_chunk; }
+    LAUNCH(c, KC_YL_PASS2, (k_yl<T, 2, false>), c->grid_fit((const void*)k_yl<T, 2, false>, nvecM), ya, c->rs, c->d_scal);
+  }
+  SIPB_CUDA_CHECK(cudaGetLastError());
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(y, S.y.p, M * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+  ProjParams<T> pp;
+  int sel[2];
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(&pp, S.pp_y.p, sizeof(pp), cudaMemcpyDeviceToHost, c->stream));
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(&sel[0], &c->d_sel->levels_run, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(&sel[1], &c->d_sel->table_valid, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(c->d_scal, 0, (slot + 3) * sizeof(double), c->stream));
+  SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));
+  // the chunk k_tie_cross settled in place: the one the quota boundary falls into (from its prefix and the counts)
+  const int g = c->max_grid();
+  int64_t cross = -1;
+  if (tie_chunk > 0 && pp.need_ties) {
+    std::vector<unsigned long long> cnt(g), base(g);
+    SIPB_CUDA_CHECK(cudaMemcpy(cnt.data(), c->d_tie_counts, g * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    SIPB_CUDA_CHECK(cudaMemcpy(base.data(), c->d_tie_base, g * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    for (int q = 0; q < g; ++q)
+      if (base[q] < pp.quota && base[q] + cnt[q] > pp.quota) cross = q;
+  }
+  if (stats) {
+    const i64 chunk = ((M + g - 1) / g + kThreads - 1) / kThreads * kThreads;     // the row partition of the tie kernels
+    const int64_t st[8] = {(int64_t)pp.key_thr, (int64_t)pp.quota, (int64_t)pp.count_eq, pp.need_ties, sel[0], sel[1],
+                           (int64_t)chunk, cross};
+    memcpy(stats, st, sizeof(st));
+  }
+  return SIPB_OK;
+}
+
 template <typename T>
 static int bench_spmv_impl(sipb_ctx* c, int ndim, const int64_t* n, int warmup, int reps, int flush_l2, double* avg_ms,
                            int64_t* alg_bytes, int form, int tiled) {
@@ -3442,6 +3609,27 @@ int sipb_cds_spmv_grid(sipb_ctx* ctx, int dtype, const int64_t* n, int nd, const
   SIPB_REQUIRE(n[0] >= 2 && n[1] >= 2 && n[2] >= 2, SIPB_E_INVALID, "grid dimensions must be >= 2");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
   DISPATCH(dtype, cds_spmv_grid_impl, ctx, n, nd, R, offsets, x, y, used_tiled);
+}
+int sipb_tile_probe(sipb_ctx* ctx, int dtype, const int64_t* n, int nd, const int64_t* offsets, const void* tab,
+                    const void* R, const void* x, const void* b, int mode, int tiled, void* y, void* r, void* p,
+                    void* x_old, double* sums, int* geom) {
+  SIPB_REQUIRE(ctx && n && offsets && x && sums, SIPB_E_INVALID, "null argument");
+  SIPB_REQUIRE((tab != nullptr) != (R != nullptr), SIPB_E_INVALID, "pass either a class table or CDS arrays");
+  SIPB_REQUIRE(mode == 1 ? y != nullptr : (mode == 2 && b && r && p && x_old), SIPB_E_INVALID,
+               "mode 1 needs y; mode 2 needs b, r, p and x_old");
+  SIPB_REQUIRE(nd >= 1 && nd <= kTileDiag, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,8]");
+  SIPB_REQUIRE(n[0] >= 2 && n[1] >= 2 && n[2] >= 2, SIPB_E_INVALID, "grid dimensions must be >= 2");
+  SIPB_REQUIRE(ctx->world <= 1, SIPB_E_UNSUPPORTED, "the probe runs on a single-GPU context");
+  SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
+  DISPATCH(dtype, tile_probe_impl, ctx, n, nd, offsets, tab, R, x, b, mode, tiled, y, r, p, x_old, sums, geom);
+}
+int sipb_select_probe(sipb_ctx* ctx, int dtype, int64_t M, const void* v, int64_t k, uint64_t guess, int path, void* y,
+                      int64_t* stats) {
+  SIPB_REQUIRE(ctx && v && y, SIPB_E_INVALID, "null argument");
+  SIPB_REQUIRE(M >= 1 && path >= 0 && path <= 2, SIPB_E_INVALID, "M >= 1 and path 0, 1 or 2");
+  SIPB_REQUIRE(ctx->world <= 1, SIPB_E_UNSUPPORTED, "the probe runs on a single-GPU context");
+  SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
+  DISPATCH(dtype, select_probe_impl, ctx, M, v, k, guess, path, y, stats);
 }
 
 }  // extern "C"

@@ -38,22 +38,24 @@ def pick(st, h):
 def select(keys, k, KB, guess=0, dbits=11, spec=True):
     """Returns (state, number of real histogram passes).  state: prefix = threshold key, k_rem = tie quota,
     count_eq = keys equal to the threshold."""
-    keys = [int(x) for x in keys]
+    keys = np.asarray(keys).astype(np.uint64)
+
+    def digit(sel, shift, w):                              # histogram of bits [shift, shift + w) of the selected keys
+        return np.bincount(((keys[sel] >> np.uint64(shift)) & np.uint64((1 << w) - 1)).astype(np.int64), minlength=BINS)
+
     st = dict(prefix=0, k_rem=k, count_eq=0, bits_left=KB, key_bits=KB, dbits=dbits)
     passes = 0
     if spec:                                              # k_yl_spec + k_sel_begin
         sh = np.zeros((SPECLEV - 1, BINS), dtype=np.int64)
-        above = 0
         g0 = guess >> (KB - SPECBITS)
-        for key in keys:
-            d0 = key >> (KB - SPECBITS)
-            above += d0 > g0
-            if d0 == g0:
-                for lv in range(1, SPECLEV):
-                    bl = KB - SPECBITS * lv
-                    w = min(bl, SPECBITS)
-                    if lv == 1 or (key >> bl) == (guess >> bl):
-                        sh[lv - 1, (key >> (bl - w)) & ((1 << w) - 1)] += 1
+        d0 = keys >> np.uint64(KB - SPECBITS)
+        above = int(np.count_nonzero(d0 > np.uint64(g0)))
+        same = d0 == np.uint64(g0)
+        for lv in range(1, SPECLEV):
+            bl = KB - SPECBITS * lv
+            w = min(bl, SPECBITS)
+            sel = same if lv == 1 else same & ((keys >> np.uint64(bl)) == np.uint64(guess >> bl))
+            sh[lv - 1] = digit(sel, bl - w, w)
         bucket = int(sh[0].sum())
         if above < k <= above + bucket:
             st.update(prefix=g0, k_rem=k - above, count_eq=bucket, bits_left=KB - SPECBITS)
@@ -68,11 +70,7 @@ def select(keys, k, KB, guess=0, dbits=11, spec=True):
             continue
         passes += 1
         w = min(dbits, bl)
-        shift, mask = bl - w, (1 << w) - 1
-        h = np.zeros(BINS, dtype=np.int64)
-        for key in keys:
-            if bl >= KB or (key >> bl) == st["prefix"]:
-                h[(key >> shift) & mask] += 1
-        pick(st, h)
+        sel = slice(None) if bl >= KB else (keys >> np.uint64(bl)) == np.uint64(st["prefix"])
+        pick(st, digit(sel, bl - w, w))
     assert st["bits_left"] == 0, st
     return st, passes
