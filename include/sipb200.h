@@ -324,6 +324,26 @@ int sipb_tile_probe(sipb_ctx* ctx, int dtype, const int64_t* n, int nd, const in
  * Unit-test entry point. */
 int sipb_select_probe(sipb_ctx* ctx, int dtype, int64_t M, const void* v, int64_t k, uint64_t guess, int path, void* y,
                       int64_t* stats);
+/* The two vector phases of PARSDMM iteration `it` (1-based) on a finalized single-GPU problem, exactly as sipb_solve
+ * runs them: the rhs gather rhs = sum_i A_i'(rho_i y_i + l_i) (rhs_compose.jl), then the y/l update of every set
+ * (update_y_l.jl:39-94) fused with the adaptation sums and snapshots (adapt_rho_gamma.jl:41-53, PARSDMM.jl:164-207),
+ * the in-loop feasibility (it % 10 == 0), the dual residual and the stop sums (PARSDMM.jl:140-145).  do_adapt is the
+ * loop's adaptation flag; it = 1 or do_adapt takes snapshots, do_adapt and it > 1 also reduces the six sums.
+ * Inputs (TF arrays of the problem's dtype): m (prod(n)), x (the CG result) and x_old (N each); per set s: l[s], y[s]
+ * (= y^k, in/out: y^{k+1} and l^{k+1} on return), y_prev[s] (= y^{k-1}), snapshots[4s..4s+3] = l_hat_0, s_0, l_0, y_0
+ * (in/out), rho[s], gamma[s]; the state a previous iteration leaves: l1_inactive_prev[s] (l1 sets: the last sum|v| <=
+ * tau), warm[2s..2s+1] (l1 warm thresholds: y update, feasibility), key_thr[s] (cardinality: previous threshold key).
+ * Outputs: rhs (N); s[s] (optional, M; sets that keep s = A x: reduction-type and sparse-operator sets); slots (512
+ * doubles: the scalar slot table, 16 per set from 0 and the global slots from 256); params[3s..] = theta, scale, fill
+ * and iparams[6s..] = key_thr, quota, count_eq, keep_all, keep_none, need_ties of each set's y-update projector;
+ * launches (SIPB_N_KERNEL_CLASSES) = launches per kernel class of this call; info[5] = {dual residual fused into the
+ * rhs gather (0/1), the iteration the r_dual slots belong to (0: none), stop sums fused (0/1), slots per set, first
+ * global slot}.  Overwrites the problem's device vectors.  SIPB_E_UNSUPPORTED on slab problems.  Unit-test entry. */
+int sipb_iter_probe(sipb_problem* pb, int it, int do_adapt, const void* m, const void* x, const void* x_old,
+                    const double* rho, const double* gamma, void* const* l, void* const* y, void* const* y_prev,
+                    void* const* snapshots, const int* l1_inactive_prev, const double* warm, const uint64_t* key_thr,
+                    void* rhs, void* const* s, double* slots, double* params, int64_t* iparams, int64_t* launches,
+                    int* info);
 
 #ifdef __cplusplus
 }

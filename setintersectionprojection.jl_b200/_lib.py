@@ -117,6 +117,9 @@ SYMBOLS = [
     ("sipb_cds_spmv_grid", _I, [_VP, _I, _PI64, _I, _VP, _PI64, _VP, _VP, _PI]),
     ("sipb_tile_probe", _I, [_VP, _I, _PI64, _I, _PI64, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP, _VP, _VP, _PD, _PI]),
     ("sipb_select_probe", _I, [_VP, _I, _I64, _VP, _I64, C.c_uint64, _I, _VP, _PI64]),
+    ("sipb_iter_probe", _I, [_VP, _I, _I, _VP, _VP, _VP, _PD, _PD, C.POINTER(_VP), C.POINTER(_VP), C.POINTER(_VP),
+                             C.POINTER(_VP), _PI, _PD, C.POINTER(C.c_uint64), _VP, C.POINTER(_VP), _PD, _PD, _PI64,
+                             _PI64, _PI]),
 ]
 
 _lib = None

@@ -2087,6 +2087,10 @@ struct Problem : sipb_problem {
 
   int solve(const void* m_h, void* x_h, void* const* l_h, void* const* y_h, const sipb_options* o,
             sipb_log* log) override;
+  // the two vector phases of one PARSDMM iteration (solve runs them around the CG; sipb_iter_probe runs them alone)
+  int rhs_phase(int i, const std::vector<T>& rho, bool fuse_rdual);
+  int yl_phase(int i, const std::vector<T>& rho, const std::vector<T>& gamma, bool do_adapt, bool fuse_stop,
+               bool fuse_rdual);
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -2149,6 +2153,193 @@ static inline double jl_maximum(const double* a, int n, int stride = 1) {
     if (v > m) m = v;
   }
   return m;
+}
+
+// rhs = sum_i A_i'(rho_i y_i + l_i) of iteration i (rhs_compose.jl); fuse_rdual: from the second iteration on the
+// gather also reduces the dual residual of iteration i-1 into the global slots 8.. (one per set)
+template <typename T>
+int Problem<T>::rhs_phase(int i, const std::vector<T>& rho, bool fuse_rdual) {
+  sipb_ctx* c = ctx;
+  const int p = (int)sets.size();
+  {
+    // sets are processed in the reference's order; runs of stencil sets go through one gather kernel each,
+    // explicit sparse operators through k_sparse_adjoint in between (rhs += A_i'(rho_i y_i + l_i))
+    const i64 ngrp = (N + 2 * Vec<T>::W - 1) / (2 * Vec<T>::W);
+    const int g_rhs = (fuse_rdual && i >= 2) ? c->grid_fit((const void*)k_rhs<T, true>, ngrp)
+                                             : c->grid_fit((const void*)k_rhs<T, false>, ngrp);
+    bool first = true;
+    int s0 = 0;
+    while (s0 < p) {
+      if (sets[s0]->is_sparse) {
+        SetT<T>& S = *sets[s0];
+        LAUNCH(c, KC_RHS, k_sparse_adjoint<T>, c->grid_for(N), S.sparse.ref(), rho[s0], (const T*)S.y.p, (const T*)S.l.p,
+               rhs.p, first ? 0 : 1);
+        first = false;
+        ++s0;
+        continue;
+      }
+      int s1 = s0;
+      while (s1 < p && !sets[s1]->is_sparse) ++s1;
+      RhsArgs<T> ra;
+      memset(&ra, 0, sizeof(ra));
+      ra.nsets = s1 - s0;
+      ra.n[0] = (unsigned)n[0]; ra.n[1] = (unsigned)n[1]; ra.n[2] = (unsigned)n[2];
+      ra.npts = npts; ra.ncols = N; ra.rhs = rhs.p;
+      ra.accumulate = first ? 0 : 1;
+      double rows = 0;
+      for (int s = s0; s < s1; ++s) {
+        ra.sets[s - s0].op = sets[s]->op;
+        ra.sets[s - s0].y = sets[s]->y.p;
+        ra.sets[s - s0].l = sets[s]->l.p;
+        ra.sets[s - s0].y_old = sets[s]->y_old.p;
+        ra.sets[s - s0].rho = rho[s];
+        rows += (double)sets[s]->M;
+      }
+      c->account(KC_RHS, ((fuse_rdual && i >= 2 ? 3 : 2) * rows + (double)N) * sizeof(T));   // y, l (, y_old) -> rhs
+      // from the second iteration on the gather also yields the dual residual of iteration i-1
+      if (fuse_rdual && i >= 2)
+        LAUNCH(c, KC_RHS, (k_rhs<T, true>), g_rhs, ra, c->rs, c->d_scal + kSlotGlobal + 8);
+      else
+        LAUNCH(c, KC_RHS, (k_rhs<T, false>), g_rhs, ra, c->rs, (double*)nullptr);
+      first = false;
+      s0 = s1;
+    }
+  }
+  return SIPB_OK;
+}
+
+// y / l update of iteration i for every set (update_y_l.jl), fused with the rho/gamma adaptation sums and snapshots,
+// the in-loop feasibility (every 10th iteration) and the stop sums; then the unfused dual residual, the slab halos of
+// y and l and, when no distance term reduced them, the stop sums (k_stop).  Results land in the scalar slots.
+template <typename T>
+int Problem<T>::yl_phase(int i, const std::vector<T>& rho, const std::vector<T>& gamma, bool do_adapt, bool fuse_stop,
+                         bool fuse_rdual) {
+  sipb_ctx* c = ctx;
+  const int p = (int)sets.size();
+  const bool feas_it = (i % 10 == 0);
+  const bool fuse_adapt = (i == 1) || do_adapt;
+  YlMultiArgs<T>& ym = yl_multi;
+  int n_multi = 0, g_multi = 1;
+  auto flush_multi = [&]() {
+    if (n_multi == 0) return;
+    const dim3 grid((unsigned)g_multi, (unsigned)n_multi);
+    if (fuse_adapt) LAUNCH(c, KC_YL_FUSED, (k_yl_multi<T, true>), grid, ym, c->rs_multi);
+    else LAUNCH(c, KC_YL_FUSED, (k_yl_multi<T, false>), grid, ym, c->rs_multi);
+    n_multi = 0;
+    g_multi = 1;
+  };
+  for (int s = 0; s < p; ++s) {
+    SetT<T>& S = *sets[s];
+    const bool is_dist = S.desc.set_kind == SIPB_SET_DISTANCE;
+    const bool want_feas = feas_it && !is_dist;
+    // copy!(y_old, y) (update_y_l.jl:64) without moving data: the two buffers trade places and the
+    // kernels read y^{k} from y_old while writing y^{k+1}
+    S.y.swap(S.y_old);
+    YlArgs<T> ya;
+    memset(&ya, 0, sizeof(ya));
+    ya.op = S.op;
+    ya.P = proj_static(S, rho[s]);
+    ya.x = x.p; ya.y = S.y.p; ya.l = S.l.p; ya.y_old = S.y_old.p; ya.s = S.s.p;
+    if (S.is_sparse) {       // s = A x by the sparse kernel; the fused kernels then apply the identity to it
+      LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(S.M), S.sparse.ref(), (const T*)x.p, S.s.p);
+      ya.x = S.s.p;
+    }
+    ya.lhat0 = S.lhat0.p; ya.s0 = S.s0.p; ya.l0 = S.l0.p; ya.y0 = S.y0.p;
+    ya.rho = rho[s]; ya.gamma = gamma[s];
+    ya.do_sums = (do_adapt && i > 1) ? 1 : 0;     // i == 1: snapshot only (all deltas are zero)
+    ya.do_snapshot = fuse_adapt ? 1 : 0;
+    const int base = s * kSlotPerSet;
+    const i64 nvecM = (S.M + Vec<T>::W - 1) / Vec<T>::W;
+    const int g = proj_is_elementwise(S.desc.set_kind)
+                      ? (fuse_adapt ? c->grid_fit((const void*)k_yl_multi<T, true>, nvecM)
+                                    : c->grid_fit((const void*)k_yl_multi<T, false>, nvecM))
+                      : c->grid_for(nvecM);
+    // streams of M rows: l in, y and l out, y_old in when relaxed or adapting, 4 snapshots in / out
+    const double rowsB = (double)S.M * sizeof(T), colsB = (double)N * sizeof(T);
+    const bool needs_yold = fuse_adapt || !(gamma[s] == (T)1);
+    const double adaptB = (fuse_adapt ? 4 : 0) * rowsB + (ya.do_sums ? 4 : 0) * rowsB;
+    if (proj_is_elementwise(S.desc.set_kind)) {
+      if (fuse_stop && is_dist) {       // the distance term also reduces the stop sums (x, m are in registers)
+        ya.x_old = x_old.p;
+        ya.stop_out = c->d_scal + kSlotGlobal;
+      }
+      c->account(KC_YL_FUSED, colsB + (3 + (needs_yold ? 1 : 0) + (ya.stop_out ? 1 : 0)) * rowsB + adaptB);
+      // element-wise sets are gathered and updated by one launch per (up to) kYlMulti sets
+      ya.want_feas = want_feas ? 1 : 0;
+      ym.a[n_multi] = ya;
+      ym.out[n_multi] = c->d_scal + base;
+      g_multi = std::max(g_multi, g);
+      if (++n_multi == kYlMulti) flush_multi();
+    } else {
+      ya.want_feas = 0;
+      // s = A x is stored only when the in-loop feasibility check reads it afterwards (every 10th iteration) or the
+      // operator is an explicit sparse matrix (its s buffer IS the input of the fused kernels)
+      ya.store_s = (want_feas && !S.is_sparse) ? 1 : 0;
+      // vector-mode cardinality on one GPU: the first levels of the radix select ride on pass 1 (k_yl_spec)
+      const bool spec = S.desc.set_kind == SIPB_SET_CARDINALITY && !sg.on && c->sel_spec;
+      // l1 ball on one GPU: pass 2 recomputes v, so pass 1 need not store it while the ball is inactive (the previous
+      // iteration's sum|v| <= tau is the guess; a wrong guess costs the gated launch below, never the result)
+      if (S.desc.set_kind == SIPB_SET_L1 && !sg.on && (c->l1_skipv == 2 || (c->l1_skipv == 1 && S.l1_inactive_prev)))
+        ya.skip_v = 1;
+      if (spec)
+        LAUNCH(c, KC_YL_PASS1, (k_yl_spec<T>), c->grid_fit((const void*)k_yl_spec<T>, nvecM), ya, c->rs,
+               c->d_scal + base + 10, &c->d_sel->spec_above, c->d_sel->spec, (const ProjParams<T>*)S.pp_y.p);
+      else
+        LAUNCH(c, KC_YL_PASS1, (k_yl<T, 1, false>), c->grid_fit((const void*)k_yl<T, 1, false>, nvecM), ya, c->rs,
+               c->d_scal + base + 10);
+      if (ya.skip_v) {
+        // v was not stored: the threshold search reads it only when sum|v| > tau.  A second launch of pass 1, gated on the
+        // device by that test (the statistics are in place), writes it then; it returns at once otherwise.
+        YlArgs<T> yb = ya;
+        yb.skip_v = 0;
+        yb.store_s = 0;
+        yb.gate = c->d_scal + base + 10;
+        yb.gate_tau = (double)(T)S.desc.max;
+        LAUNCH(c, KC_YL_PASS1, (k_yl<T, 1, false>), c->grid_fit((const void*)k_yl<T, 1, false>, nvecM), yb, c->rs,
+               c->d_scal + base + 13);
+      }
+      // pass 1: x, l (, y_old) -> v (, s);   pass 2: v, x, l (, y_old) -> y, l
+      // (an l1 set's pass 2 recomputes v instead of reading it; pass 1 skips the store while the ball is inactive)
+      const int l1set = S.desc.set_kind == SIPB_SET_L1 ? 1 : 0;
+      c->account(KC_YL_PASS1, colsB + (2 - ya.skip_v + (!(gamma[s] == (T)1) ? 1 : 0) + ya.store_s) * rowsB);
+      c->account(KC_YL_PASS2, colsB + (4 - l1set + (needs_yold ? 1 : 0)) * rowsB + adaptB);
+      i64 tie_chunk = 0;
+      const bool defer = S.desc.set_kind == SIPB_SET_CARDINALITY && !sg.on && c->sel_spec;
+      int rc = projector_params(S, S.y.p, base + 10, S.pp_y.p, S.warm.p, true, spec, defer ? &tie_chunk : nullptr);
+      if (rc) return rc;
+      ya.dyn = S.pp_y.p;
+      if (tie_chunk > 0) { ya.P.tie_base = c->d_tie_base; ya.P.tie_chunk = tie_chunk; }
+      if (fuse_adapt)
+        LAUNCH(c, KC_YL_PASS2, (k_yl<T, 2, true>), c->grid_fit((const void*)k_yl<T, 2, true>, nvecM), ya, c->rs,
+               c->d_scal + base);
+      else
+        LAUNCH(c, KC_YL_PASS2, (k_yl<T, 2, false>), c->grid_fit((const void*)k_yl<T, 2, false>, nvecM), ya, c->rs,
+               c->d_scal + base);
+      if (want_feas) {
+        rc = feasibility_of(S, S.s.p, base + 1, true);
+        if (rc) return rc;
+      }
+    }
+  }
+  flush_multi();
+  if (!fuse_rdual) {
+    for (int s = 0; s < p; ++s) {
+      SetT<T>& S = *sets[s];
+      if (S.is_sparse)
+        LAUNCH(c, KC_RDUAL, k_sparse_rdual<T>, c->grid_for(N), S.sparse.ref(), (const T*)S.y.p, (const T*)S.y_old.p, c->rs,
+               c->d_scal + s * kSlotPerSet + 3);
+      else
+        LAUNCH(c, KC_RDUAL, k_rdual<T>, c->grid_for((npts + Vec<T>::W - 1) / Vec<T>::W), S.op, (const T*)S.y.p,
+               (const T*)S.y_old.p, c->rs, c->d_scal + s * kSlotPerSet + 3);
+    }
+  }
+  { int rc = exchange_yl_halos(); if (rc) return rc; }   // slabs: halo planes for the next rhs gather
+  if (!fuse_stop) {
+    LAUNCH(c, KC_STOP, k_stop<T>, c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), N, npts, minkowski ? 1 : 0, (const T*)x.p,
+           (const T*)x_old.p, (const T*)m.p, c->rs, c->d_scal + kSlotGlobal);
+    c->account(KC_STOP, 3.0 * N * sizeof(T));                            // x, x_old, m
+  }
+  return SIPB_OK;
 }
 
 // =============================================================================================
@@ -2354,50 +2545,7 @@ int Problem<T>::solve(const void* m_h, void* x_h, void* const* l_h, void* const*
   const int it_limit = o->fixed_iterations > 0 ? std::min(o->fixed_iterations, maxit) : maxit;
   for (int i = 1; i <= it_limit; ++i) {
     // ---------------- rhs (rhs_compose.jl) ---------------------------------------------------
-    {
-      // sets are processed in the reference's order; runs of stencil sets go through one gather kernel each,
-      // explicit sparse operators through k_sparse_adjoint in between (rhs += A_i'(rho_i y_i + l_i))
-      const i64 ngrp = (N + 2 * Vec<T>::W - 1) / (2 * Vec<T>::W);
-      const int g_rhs = (fuse_rdual && i >= 2) ? c->grid_fit((const void*)k_rhs<T, true>, ngrp)
-                                               : c->grid_fit((const void*)k_rhs<T, false>, ngrp);
-      bool first = true;
-      int s0 = 0;
-      while (s0 < p) {
-        if (sets[s0]->is_sparse) {
-          SetT<T>& S = *sets[s0];
-          LAUNCH(c, KC_RHS, k_sparse_adjoint<T>, c->grid_for(N), S.sparse.ref(), rho[s0], (const T*)S.y.p, (const T*)S.l.p,
-                 rhs.p, first ? 0 : 1);
-          first = false;
-          ++s0;
-          continue;
-        }
-        int s1 = s0;
-        while (s1 < p && !sets[s1]->is_sparse) ++s1;
-        RhsArgs<T> ra;
-        memset(&ra, 0, sizeof(ra));
-        ra.nsets = s1 - s0;
-        ra.n[0] = (unsigned)n[0]; ra.n[1] = (unsigned)n[1]; ra.n[2] = (unsigned)n[2];
-        ra.npts = npts; ra.ncols = N; ra.rhs = rhs.p;
-        ra.accumulate = first ? 0 : 1;
-        double rows = 0;
-        for (int s = s0; s < s1; ++s) {
-          ra.sets[s - s0].op = sets[s]->op;
-          ra.sets[s - s0].y = sets[s]->y.p;
-          ra.sets[s - s0].l = sets[s]->l.p;
-          ra.sets[s - s0].y_old = sets[s]->y_old.p;
-          ra.sets[s - s0].rho = rho[s];
-          rows += (double)sets[s]->M;
-        }
-        c->account(KC_RHS, ((fuse_rdual && i >= 2 ? 3 : 2) * rows + (double)N) * sizeof(T));   // y, l (, y_old) -> rhs
-        // from the second iteration on the gather also yields the dual residual of iteration i-1
-        if (fuse_rdual && i >= 2)
-          LAUNCH(c, KC_RHS, (k_rhs<T, true>), g_rhs, ra, c->rs, c->d_scal + kSlotGlobal + 8);
-        else
-          LAUNCH(c, KC_RHS, (k_rhs<T, false>), g_rhs, ra, c->rs, (double*)nullptr);
-        first = false;
-        s0 = s1;
-      }
-    }
+    { int rc = rhs_phase(i, rho, fuse_rdual); if (rc) return rc; }
     phase_end(1);
     // ---------------- x-minimisation (argmin_x.jl + cg.jl) -----------------------------------
     int cg_it = 0, cg_flag = 0;
@@ -2420,128 +2568,7 @@ int Problem<T>::solve(const void* m_h, void* x_h, void* const* l_h, void* const*
     // rho/gamma adaptation is fused into the y/l kernels: the flags are known before the update; if
     // stop_PARSDMM switches adaptation off in this very iteration the sums are simply discarded
     const bool do_adapt = (adjust_rho || adjust_gamma) && (i % rho_update_frequency == 0);
-    const bool fuse_adapt = (i == 1) || do_adapt;
-    YlMultiArgs<T>& ym = yl_multi;
-    int n_multi = 0, g_multi = 1;
-    auto flush_multi = [&]() {
-      if (n_multi == 0) return;
-      const dim3 grid((unsigned)g_multi, (unsigned)n_multi);
-      if (fuse_adapt) LAUNCH(c, KC_YL_FUSED, (k_yl_multi<T, true>), grid, ym, c->rs_multi);
-      else LAUNCH(c, KC_YL_FUSED, (k_yl_multi<T, false>), grid, ym, c->rs_multi);
-      n_multi = 0;
-      g_multi = 1;
-    };
-    for (int s = 0; s < p; ++s) {
-      SetT<T>& S = *sets[s];
-      const bool is_dist = S.desc.set_kind == SIPB_SET_DISTANCE;
-      const bool want_feas = feas_it && !is_dist;
-      // copy!(y_old, y) (update_y_l.jl:64) without moving data: the two buffers trade places and the
-      // kernels read y^{k} from y_old while writing y^{k+1}
-      S.y.swap(S.y_old);
-      YlArgs<T> ya;
-      memset(&ya, 0, sizeof(ya));
-      ya.op = S.op;
-      ya.P = proj_static(S, rho[s]);
-      ya.x = x.p; ya.y = S.y.p; ya.l = S.l.p; ya.y_old = S.y_old.p; ya.s = S.s.p;
-      if (S.is_sparse) {       // s = A x by the sparse kernel; the fused kernels then apply the identity to it
-        LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(S.M), S.sparse.ref(), (const T*)x.p, S.s.p);
-        ya.x = S.s.p;
-      }
-      ya.lhat0 = S.lhat0.p; ya.s0 = S.s0.p; ya.l0 = S.l0.p; ya.y0 = S.y0.p;
-      ya.rho = rho[s]; ya.gamma = gamma[s];
-      ya.do_sums = (do_adapt && i > 1) ? 1 : 0;     // i == 1: snapshot only (all deltas are zero)
-      ya.do_snapshot = fuse_adapt ? 1 : 0;
-      const int base = s * kSlotPerSet;
-      const i64 nvecM = (S.M + Vec<T>::W - 1) / Vec<T>::W;
-      const int g = proj_is_elementwise(S.desc.set_kind)
-                        ? (fuse_adapt ? c->grid_fit((const void*)k_yl_multi<T, true>, nvecM)
-                                      : c->grid_fit((const void*)k_yl_multi<T, false>, nvecM))
-                        : c->grid_for(nvecM);
-      // streams of M rows: l in, y and l out, y_old in when relaxed or adapting, 4 snapshots in / out
-      const double rowsB = (double)S.M * sizeof(T), colsB = (double)N * sizeof(T);
-      const bool needs_yold = fuse_adapt || !(gamma[s] == (T)1);
-      const double adaptB = (fuse_adapt ? 4 : 0) * rowsB + (ya.do_sums ? 4 : 0) * rowsB;
-      if (proj_is_elementwise(S.desc.set_kind)) {
-        if (fuse_stop && is_dist) {       // the distance term also reduces the stop sums (x, m are in registers)
-          ya.x_old = x_old.p;
-          ya.stop_out = c->d_scal + kSlotGlobal;
-        }
-        c->account(KC_YL_FUSED, colsB + (3 + (needs_yold ? 1 : 0) + (ya.stop_out ? 1 : 0)) * rowsB + adaptB);
-        // element-wise sets are gathered and updated by one launch per (up to) kYlMulti sets
-        ya.want_feas = want_feas ? 1 : 0;
-        ym.a[n_multi] = ya;
-        ym.out[n_multi] = c->d_scal + base;
-        g_multi = std::max(g_multi, g);
-        if (++n_multi == kYlMulti) flush_multi();
-      } else {
-        ya.want_feas = 0;
-        // s = A x is stored only when the in-loop feasibility check reads it afterwards (every 10th iteration) or the
-        // operator is an explicit sparse matrix (its s buffer IS the input of the fused kernels)
-        ya.store_s = (want_feas && !S.is_sparse) ? 1 : 0;
-        // vector-mode cardinality on one GPU: the first levels of the radix select ride on pass 1 (k_yl_spec)
-        const bool spec = S.desc.set_kind == SIPB_SET_CARDINALITY && !sg.on && c->sel_spec;
-        // l1 ball on one GPU: pass 2 recomputes v, so pass 1 need not store it while the ball is inactive (the previous
-        // iteration's sum|v| <= tau is the guess; a wrong guess costs the gated launch below, never the result)
-        if (S.desc.set_kind == SIPB_SET_L1 && !sg.on && (c->l1_skipv == 2 || (c->l1_skipv == 1 && S.l1_inactive_prev)))
-          ya.skip_v = 1;
-        if (spec)
-          LAUNCH(c, KC_YL_PASS1, (k_yl_spec<T>), c->grid_fit((const void*)k_yl_spec<T>, nvecM), ya, c->rs,
-                 c->d_scal + base + 10, &c->d_sel->spec_above, c->d_sel->spec, (const ProjParams<T>*)S.pp_y.p);
-        else
-          LAUNCH(c, KC_YL_PASS1, (k_yl<T, 1, false>), c->grid_fit((const void*)k_yl<T, 1, false>, nvecM), ya, c->rs,
-                 c->d_scal + base + 10);
-        if (ya.skip_v) {
-          // v was not stored: the threshold search reads it only when sum|v| > tau.  A second launch of pass 1, gated on the
-          // device by that test (the statistics are in place), writes it then; it returns at once otherwise.
-          YlArgs<T> yb = ya;
-          yb.skip_v = 0;
-          yb.store_s = 0;
-          yb.gate = c->d_scal + base + 10;
-          yb.gate_tau = (double)(T)S.desc.max;
-          LAUNCH(c, KC_YL_PASS1, (k_yl<T, 1, false>), c->grid_fit((const void*)k_yl<T, 1, false>, nvecM), yb, c->rs,
-                 c->d_scal + base + 13);
-        }
-        // pass 1: x, l (, y_old) -> v (, s);   pass 2: v, x, l (, y_old) -> y, l
-        // (an l1 set's pass 2 recomputes v instead of reading it; pass 1 skips the store while the ball is inactive)
-        const int l1set = S.desc.set_kind == SIPB_SET_L1 ? 1 : 0;
-        c->account(KC_YL_PASS1, colsB + (2 - ya.skip_v + (!(gamma[s] == (T)1) ? 1 : 0) + ya.store_s) * rowsB);
-        c->account(KC_YL_PASS2, colsB + (4 - l1set + (needs_yold ? 1 : 0)) * rowsB + adaptB);
-        i64 tie_chunk = 0;
-        const bool defer = S.desc.set_kind == SIPB_SET_CARDINALITY && !sg.on && c->sel_spec;
-        int rc = projector_params(S, S.y.p, base + 10, S.pp_y.p, S.warm.p, true, spec, defer ? &tie_chunk : nullptr);
-        if (rc) return rc;
-        ya.dyn = S.pp_y.p;
-        if (tie_chunk > 0) { ya.P.tie_base = c->d_tie_base; ya.P.tie_chunk = tie_chunk; }
-        if (fuse_adapt)
-          LAUNCH(c, KC_YL_PASS2, (k_yl<T, 2, true>), c->grid_fit((const void*)k_yl<T, 2, true>, nvecM), ya, c->rs,
-                 c->d_scal + base);
-        else
-          LAUNCH(c, KC_YL_PASS2, (k_yl<T, 2, false>), c->grid_fit((const void*)k_yl<T, 2, false>, nvecM), ya, c->rs,
-                 c->d_scal + base);
-        if (want_feas) {
-          rc = feasibility_of(S, S.s.p, base + 1, true);
-          if (rc) return rc;
-        }
-      }
-    }
-    flush_multi();
-    if (!fuse_rdual) {
-      for (int s = 0; s < p; ++s) {
-        SetT<T>& S = *sets[s];
-        if (S.is_sparse)
-          LAUNCH(c, KC_RDUAL, k_sparse_rdual<T>, c->grid_for(N), S.sparse.ref(), (const T*)S.y.p, (const T*)S.y_old.p, c->rs,
-                 c->d_scal + s * kSlotPerSet + 3);
-        else
-          LAUNCH(c, KC_RDUAL, k_rdual<T>, c->grid_for((npts + Vec<T>::W - 1) / Vec<T>::W), S.op, (const T*)S.y.p,
-                 (const T*)S.y_old.p, c->rs, c->d_scal + s * kSlotPerSet + 3);
-      }
-    }
-    { int rc = exchange_yl_halos(); if (rc) return rc; }   // slabs: halo planes for the next rhs gather
-    if (!fuse_stop) {
-      LAUNCH(c, KC_STOP, k_stop<T>, c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), N, npts, minkowski ? 1 : 0, (const T*)x.p,
-             (const T*)x_old.p, (const T*)m.p, c->rs, c->d_scal + kSlotGlobal);
-      c->account(KC_STOP, 3.0 * N * sizeof(T));                            // x, x_old, m
-    }
+    { int rc = yl_phase(i, rho, gamma, do_adapt, fuse_stop, fuse_rdual); if (rc) return rc; }
     { int rc = ctx_sync_scalars(c, true); if (rc) return rc; }
     if (c->p2p) SIPB_REQUIRE(*c->h_p2p_err == 0, SIPB_E_NCCL, "peer-memory collective timed out (a rank stopped participating)");
     SIPB_REQUIRE(!c->h_l1->failed, SIPB_E_STATE, "l1 threshold search did not converge");
@@ -3464,6 +3491,89 @@ static int select_probe_impl(sipb_ctx* c, int64_t M, const void* v, int64_t k, u
   return SIPB_OK;
 }
 
+// One PARSDMM iteration's vector phases on a finalized single-GPU problem (unit tests): the caller's state is uploaded
+// as the loop would leave it before iteration `it` (x stands for the CG's result), then rhs_phase and yl_phase run
+// with the flags solve derives for that iteration.  Overwrites the problem's device vectors.
+template <typename T>
+static int iter_probe_impl(Problem<T>* P, int it, int do_adapt, const void* m_h, const void* x_h, const void* x_old_h,
+                           const double* rho_d, const double* gamma_d, void* const* l_h, void* const* y_h,
+                           void* const* y_prev_h, void* const* snap_h, const int* l1_inactive_prev, const double* warm,
+                           const uint64_t* key_thr, void* rhs_h, void* const* s_h, double* slots, double* params,
+                           int64_t* iparams, int64_t* launches, int* info) {
+  sipb_ctx* c = P->ctx;
+  const int p = (int)P->sets.size();
+  const i64 N = P->N, npts = P->npts;
+  c->reset_accounting();
+  c->profile = false;
+  std::vector<T> rho(p), gamma(p);
+  for (int s = 0; s < p; ++s) { rho[s] = (T)rho_d[s]; gamma[s] = (T)gamma_d[s]; }
+  auto up = [&](T* d, const void* h, i64 n) { return cudaMemcpyAsync(d, h, n * sizeof(T), cudaMemcpyHostToDevice, c->stream); };
+  auto down = [&](void* h, const T* d, i64 n) { return cudaMemcpyAsync(h, d, n * sizeof(T), cudaMemcpyDeviceToHost, c->stream); };
+  // m as solve uploads it ([m; 0] for Minkowski); the resident copy no longer belongs to a solve
+  SIPB_CUDA_CHECK(up(P->m.p, m_h, npts));
+  if (P->minkowski) SIPB_CUDA_CHECK(cudaMemsetAsync(P->m.p + npts, 0, npts * sizeof(T), c->stream));
+  P->m_resident = false;
+  SIPB_CUDA_CHECK(up(P->x.p, x_h, N));
+  SIPB_CUDA_CHECK(up(P->x_old.p, x_old_h, N));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(c->d_scal, 0, kScalSlots * sizeof(double), c->stream));
+  SIPB_CUDA_CHECK(cudaMemsetAsync(c->d_l1, 0, sizeof(L1State), c->stream));
+  bool any_sparse = false;
+  for (int s = 0; s < p; ++s) {
+    SetT<T>& S = *P->sets[s];
+    any_sparse = any_sparse || S.is_sparse;
+    SIPB_CUDA_CHECK(up(S.l.p, l_h[s], S.M));
+    SIPB_CUDA_CHECK(up(S.y.p, y_h[s], S.M));
+    SIPB_CUDA_CHECK(up(S.y_old.p, y_prev_h[s], S.M));
+    T* snaps[4] = {S.lhat0.p, S.s0.p, S.l0.p, S.y0.p};
+    for (int q = 0; q < 4; ++q) SIPB_CUDA_CHECK(up(snaps[q], snap_h[4 * s + q], S.M));
+    if (S.s.p) SIPB_CUDA_CHECK(cudaMemsetAsync(S.s.p, 0, S.M * sizeof(T), c->stream));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(S.warm.p, warm + 2 * s, 2 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    const unsigned long long k64 = key_thr[s];
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(&S.pp_y.p->key_thr, &k64, sizeof(k64), cudaMemcpyHostToDevice, c->stream));
+    S.l1_inactive_prev = l1_inactive_prev[s] != 0;
+  }
+  SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));   // the host staging above is pageable / on the stack
+  // the flags of Problem::solve at iteration `it`
+  const bool fuse_stop = !P->feas_only && !P->minkowski && getenv("SIPB_FUSE_STOP_OFF") == nullptr;
+  const bool fuse_rdual = p <= kRdualSets && !any_sparse;
+  int rc = P->rhs_phase(it, rho, fuse_rdual);
+  if (rc) return rc;
+  rc = P->yl_phase(it, rho, gamma, do_adapt != 0, fuse_stop, fuse_rdual);
+  if (rc) return rc;
+  rc = ctx_sync_scalars(c, true);
+  if (rc) return rc;
+  SIPB_REQUIRE(!c->h_l1->failed, SIPB_E_STATE, "l1 threshold search did not converge");
+  SIPB_CUDA_CHECK(down(rhs_h, P->rhs.p, N));
+  std::vector<ProjParams<T>> pp(p);
+  for (int s = 0; s < p; ++s) {
+    SetT<T>& S = *P->sets[s];
+    SIPB_CUDA_CHECK(down(l_h[s], S.l.p, S.M));
+    SIPB_CUDA_CHECK(down(y_h[s], S.y.p, S.M));
+    const T* snaps[4] = {S.lhat0.p, S.s0.p, S.l0.p, S.y0.p};
+    for (int q = 0; q < 4; ++q) SIPB_CUDA_CHECK(down(snap_h[4 * s + q], snaps[q], S.M));
+    if (s_h && s_h[s] && S.s.p) SIPB_CUDA_CHECK(down(s_h[s], S.s.p, S.M));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(&pp[s], S.pp_y.p, sizeof(ProjParams<T>), cudaMemcpyDeviceToHost, c->stream));
+  }
+  SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));
+  memcpy(slots, c->h_scal, kScalSlots * sizeof(double));
+  for (int s = 0; s < p; ++s) {
+    const double dp[3] = {(double)pp[s].theta, (double)pp[s].scale, (double)pp[s].fill};
+    const int64_t ip[6] = {(int64_t)pp[s].key_thr, (int64_t)pp[s].quota, (int64_t)pp[s].count_eq, pp[s].keep_all,
+                           pp[s].keep_none, pp[s].need_ties};
+    memcpy(params + 3 * s, dp, sizeof(dp));
+    memcpy(iparams + 6 * s, ip, sizeof(ip));
+  }
+  for (int q = 0; q < SIPB_N_KERNEL_CLASSES; ++q) launches[q] = c->launches[q];
+  // the r_dual slots: fused, the rhs gather of `it` reduced iteration it-1 into the global slots (none at it = 1);
+  // unfused, k_rdual reduced iteration `it` into each set's slot 3
+  info[0] = fuse_rdual ? 1 : 0;
+  info[1] = fuse_rdual ? it - 1 : it;
+  info[2] = fuse_stop ? 1 : 0;
+  info[3] = kSlotPerSet;
+  info[4] = kSlotGlobal;
+  return SIPB_OK;
+}
+
 template <typename T>
 static int bench_spmv_impl(sipb_ctx* c, int ndim, const int64_t* n, int warmup, int reps, int flush_l2, double* avg_ms,
                            int64_t* alg_bytes, int form, int tiled) {
@@ -3630,6 +3740,29 @@ int sipb_select_probe(sipb_ctx* ctx, int dtype, int64_t M, const void* v, int64_
   SIPB_REQUIRE(ctx->world <= 1, SIPB_E_UNSUPPORTED, "the probe runs on a single-GPU context");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
   DISPATCH(dtype, select_probe_impl, ctx, M, v, k, guess, path, y, stats);
+}
+int sipb_iter_probe(sipb_problem* pb, int it, int do_adapt, const void* m, const void* x, const void* x_old,
+                    const double* rho, const double* gamma, void* const* l, void* const* y, void* const* y_prev,
+                    void* const* snapshots, const int* l1_inactive_prev, const double* warm, const uint64_t* key_thr,
+                    void* rhs, void* const* s, double* slots, double* params, int64_t* iparams, int64_t* launches,
+                    int* info) {
+  SIPB_REQUIRE(pb && m && x && x_old && rho && gamma && l && y && y_prev && snapshots && l1_inactive_prev && warm &&
+                   key_thr && rhs && slots && params && iparams && launches && info,
+               SIPB_E_INVALID, "null argument");
+  SIPB_REQUIRE(it >= 1, SIPB_E_INVALID, "it must be >= 1");
+  SIPB_CUDA_CHECK(cudaSetDevice(pb->ctx->device));
+  if (pb->dtype == SIPB_F32) {
+    auto* P = dynamic_cast<Problem<float>*>(pb);
+    SIPB_REQUIRE(P && P->finalized, SIPB_E_STATE, "problem not finalized");
+    SIPB_REQUIRE(!P->sg.on, SIPB_E_UNSUPPORTED, "the probe runs on a single-GPU problem (no slabs)");
+    return iter_probe_impl<float>(P, it, do_adapt, m, x, x_old, rho, gamma, l, y, y_prev, snapshots, l1_inactive_prev,
+                                  warm, key_thr, rhs, s, slots, params, iparams, launches, info);
+  }
+  auto* P = dynamic_cast<Problem<double>*>(pb);
+  SIPB_REQUIRE(P && P->finalized, SIPB_E_STATE, "problem not finalized");
+  SIPB_REQUIRE(!P->sg.on, SIPB_E_UNSUPPORTED, "the probe runs on a single-GPU problem (no slabs)");
+  return iter_probe_impl<double>(P, it, do_adapt, m, x, x_old, rho, gamma, l, y, y_prev, snapshots, l1_inactive_prev,
+                                 warm, key_thr, rhs, s, slots, params, iparams, launches, info);
 }
 
 }  // extern "C"
