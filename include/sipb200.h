@@ -102,7 +102,9 @@ typedef struct sipb_set_desc {
   int32_t fiber_axis;      /* fiber modes (app_mode ("fiber","x"|"y"|"z")): 0, 1 or 2 — axis of the transform-domain grid */
   int32_t reserved;
   int64_t td_n[3];         /* fiber modes: set_Prop.TD_n[i], the transform-domain grid (third entry 1 in 2-D)  */
-  const sipb_sparse* sparse;  /* SIPB_OP_SPARSE: the matrix (copied to the device by sipb_problem_add_set), else NULL */
+  const sipb_sparse* sparse;  /* SIPB_OP_SPARSE: the matrix A with prod(n) columns (copied to the device by
+                                 sipb_problem_add_set), else NULL; in a Minkowski problem block_mode places it as
+                                 [A 0], [0 A] or [A A].  Single GPU, matrix/tensor mode. */
 } sipb_set_desc;
 
 /* Mirror of PARSDMM_options (SetIntersectionProjection.jl:110-128) after convert_options!. */
@@ -213,10 +215,13 @@ int sipb_problem_create(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, co
 /* sets must be added in TD_OP order; the distance term (SIPB_SET_DISTANCE) last. */
 int sipb_problem_add_set(sipb_problem* pb, const sipb_set_desc* desc);
 /* AtA[i] in CDS form exactly as mat2CDS (mat2CDS.jl:7-32) returns it: R is column-major
- * [rows x nd] host TF, offsets int64[nd] ascending. */
+ * [rows x nd] host TF, offsets int64[nd] ascending, 1 <= nd <= 999 (the reference's 999 x 99 offset table,
+ * PARSDMM_initialize.jl:217-221).  A Q of more than 32 diagonals (custom operators) is held as CDS arrays and
+ * needs a single GPU. */
 int sipb_problem_set_ata(sipb_problem* pb, int set_index, const void* R, int64_t rows,
                          const int64_t* offsets, int nd);
-/* AtA[i] as one row per stencil class instead of the [rows x nd] array: tab is host TF[54][nd], tab[cls*nd + j] =
+/* AtA[i] as one row per stencil class instead of the [rows x nd] array (nd <= 32, and Q <= 32 diagonals):
+ * tab is host TF[54][nd], tab[cls*nd + j] =
  * AtA[r, r + offsets[j]] for any row r of class cls = ((half*3 + c(k))*3 + c(j))*3 + c(i), c = 0 / 1 / 2 for the
  * first / an interior / the last index of the axis (half = second Minkowski half).  Every A'A the reference builds
  * from get_TD_operator.jl has this structure; passing the table skips forming, uploading and verifying the array
@@ -270,10 +275,11 @@ int sipb_solve_batch(sipb_problem* const* pbs, int B, const void* const* m, void
                      void* const* const* y, const sipb_options* opt, sipb_log* const* logs, int* rcs);
 
 /* ---- unit entry points (host pointers; used by the parity tests and micro-benchmarks) ------ */
-/* y = A*x for A in CDS form: replaces Ax_CDS_MT / CDS_MVp_MT (argmin_x.jl:72-78, CDS_MVp_MT.jl:9-25) */
+/* y = A*x for A in CDS form: replaces Ax_CDS_MT / CDS_MVp_MT (argmin_x.jl:72-78, CDS_MVp_MT.jl:9-25).
+ * 1 <= nd <= 999; each row accumulates in the order of `offsets`. */
 int sipb_cds_spmv(sipb_ctx* ctx, int dtype, int64_t N, int nd, const void* R, const int64_t* offsets,
                   const void* x, void* y);
-/* cg(A,b;tol,maxIter,x) with A in CDS form (cg.jl:44-128).  x in/out. */
+/* cg(A,b;tol,maxIter,x) with A in CDS form (cg.jl:44-128), 1 <= nd <= 999.  x in/out. */
 int sipb_cds_cg(sipb_ctx* ctx, int dtype, int64_t N, int nd, const void* R, const int64_t* offsets,
                 const void* b, void* x, double tol, int max_iter, int* flag, double* relres, int* iters);
 /* in-place projector / prox on a host vector (P_sub[i](v), get_projector.jl). `m_vec` only for
@@ -286,7 +292,12 @@ int sipb_op_apply(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, const do
 int sipb_op_rows(int ndim, const int64_t* n, int op_kind, int64_t* rows);
 /* the same for an explicit sparse operator (SIPB_OP_SPARSE) */
 int sipb_sparse_apply(sipb_ctx* ctx, int dtype, const sipb_sparse* A, int adjoint, const void* in, void* out);
-/* Q += alpha*B on matching diagonals (CDS_scaled_add!.jl:8-26). */
+/* ... and for its Minkowski block form B = A, [A 0], [0 A] or [A A] (block_mode, SIPB_BLOCK_*): s = B*x (x: 2N
+ * entries unless PLAIN) or t = B'*v (t: 2N entries unless PLAIN), folded as SparseArrays folds the hcat matrix
+ * (row r of [A A]: A's entries on x[0:N), then the same entries on x[N:2N)). */
+int sipb_sparse_apply_block(sipb_ctx* ctx, int dtype, const sipb_sparse* A, int block_mode, int adjoint,
+                            const void* in, void* out);
+/* Q += alpha*B on matching diagonals (CDS_scaled_add!.jl:8-26); B has at most 999 diagonals. */
 int sipb_cds_scaled_add(sipb_ctx* ctx, int dtype, int64_t N, int nd_a, void* A, const int64_t* a_offsets,
                         int nd_b, const void* B, const int64_t* b_offsets, double alpha);
 /* micro-benchmark: device-resident CDS SpMV(+dot) on synthetic data, CUDA-event timed;
@@ -295,7 +306,8 @@ int sipb_bench_spmv(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, int wa
                     int flush_l2, double* avg_ms, int64_t* algorithmic_bytes);
 
 /* the same with a choice of matrix form (0 = CDS arrays, (nd+2)*N*s algorithmic bytes; 1 = stencil-class tables,
- * 2*N*s) and of kernel (tiled = 1: the TMA-staged plane sweep of spmv_tile.cuh; 0: the generic grid-stride kernel) */
+ * 2*N*s; 2 = CDS arrays with the 125 diagonals of a 27-point stencil's A'A through the wide kernel, 127*N*s, 3-D only,
+ * `tiled` ignored) and of kernel (tiled = 1: the TMA-staged plane sweep of spmv_tile.cuh; 0: the generic grid-stride kernel) */
 int sipb_bench_spmv2(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, int warmup, int reps, int flush_l2,
                      int form, int tiled, double* avg_ms, int64_t* algorithmic_bytes);
 /* y = A*x (CDS_MVp_MT.jl:9-25) for a CDS matrix living on a 3-D grid: takes the tiled kernel when the offsets are a

@@ -273,9 +273,28 @@ function PARSDMM_precompute_distribute_Minkowski(TD_OP_c1, TD_OP_c2, TD_OP_sum, 
         append!(getfield(set_Prop, f), deepcopy(getfield(other, f)))
     end
     TD_OP = vcat(TD_OP_c1, TD_OP_c2, TD_OP_sum)
-    any(op -> op.kind == "custom", TD_OP) && error("custom operators inside generalized Minkowski sets are not on the device path")
-    AtA = Any[class_table(op, comp_grid) for op in TD_OP]
-    for i in eachindex(TD_OP); set_Prop.AtA_offsets[i] = AtA[i].offsets; end
+    if any(op -> op.kind == "custom", TD_OP)
+        # a custom operator has no class table: CDS arrays for every set, mat2CDS of the 2N x 2N block matrices of
+        # A'A formed like the reference (PARSDMM_precompute_distribute_Minkowski.jl:32-74,91-101,123-131)
+        N = prod(TD_OP[1].n[1:TD_OP[1].ndim])
+        Z = spzeros(TF, N, N)
+        AtA = Vector{Any}(undef, length(TD_OP))
+        for (i, op) in enumerate(TD_OP)
+            if op.kind == "custom"
+                B = op.A' * op.A
+            elseif op.kind == "identity"
+                B = spdiagm(0 => ones(TF, N))
+            else
+                A = SIP.get_TD_operator(comp_grid, op.kind, TF)[1]
+                B = A' * A
+            end
+            M = op.block_mode == BLOCK_LEFT ? [B Z; Z Z] : (op.block_mode == BLOCK_RIGHT ? [Z Z; Z B] : [B B; B B])
+            (AtA[i], set_Prop.AtA_offsets[i]) = SIP.mat2CDS(M)
+        end
+    else
+        AtA = Any[class_table(op, comp_grid) for op in TD_OP]
+    end
+    for i in eachindex(TD_OP); AtA[i] isa ClassTable && (set_Prop.AtA_offsets[i] = AtA[i].offsets); end
     y = [zeros(TF, size(op, 1)) for op in TD_OP]; l = deepcopy(y)
     return TD_OP, set_Prop, AtA, l, y
 end

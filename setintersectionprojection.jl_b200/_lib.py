@@ -111,6 +111,7 @@ SYMBOLS = [
     ("sipb_op_apply", _I, [_VP, _I, _I, _PI64, _PD, _I, _I, _I, _VP, _VP]),
     ("sipb_op_rows", _I, [_I, _PI64, _I, _PI64]),
     ("sipb_sparse_apply", _I, [_VP, _I, C.POINTER(Sparse), _I, _VP, _VP]),
+    ("sipb_sparse_apply_block", _I, [_VP, _I, C.POINTER(Sparse), _I, _I, _VP, _VP]),
     ("sipb_cds_scaled_add", _I, [_VP, _I, _I64, _I, _VP, _PI64, _I, _VP, _PI64, _D]),
     ("sipb_bench_spmv", _I, [_VP, _I, _I, _PI64, _I, _I, _I, _PD, _PI64]),
     ("sipb_bench_spmv2", _I, [_VP, _I, _I, _PI64, _I, _I, _I, _I, _I, _PD, _PI64]),

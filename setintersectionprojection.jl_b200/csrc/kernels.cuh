@@ -4,6 +4,8 @@
 //   k_spmv_tile       (spmv_tile.cuh) the same SpMV / CG prologue for 3-D stencils as a plane sweep with TMA-staged tiles
 //   k_spmv            CDS_MVp_MT.jl:9-25 + Ax_CDS_MT (argmin_x.jl:72-78) [+ dot(p,Ap), cg.jl:88]; Q as CDS arrays
 //                     or as verified stencil-class tables (k_class_extract / k_class_verify / k_class_axpy)
+//   k_spmv_wide       the same SpMV for Q with more than kMaxDiag diagonals (custom operators), offsets in device memory;
+//   k_cg_init_wide      k_cg_init likewise;  k_cds_axpy_wide  the Q update on all diagonals of one A'A in one launch
 //   k_cg_init         argmin_x.jl:33-37 + cg.jl:47-76   (one SpMV instead of the reference's two)
 //   k_cg_xr / k_cg_p  cg.jl:86-114
 //   k_rhs             rhs_compose.jl:24-36 (+ the dual residual of the previous iteration, update_y_l.jl:82-84)
@@ -22,7 +24,8 @@
 
 namespace sipb {
 
-constexpr int kMaxDiag = 32;   // max diagonals of Q handled by the SpMV kernels
+constexpr int kMaxDiag = 32;   // max diagonals of Q handled by k_spmv / k_cg_init (wider Q: the *_wide kernels)
+constexpr int kMaxDiagWide = 999;   // max diagonals of one A'A (the 999 x 99 offset table of PARSDMM_initialize.jl:217-221)
 constexpr int kMaxSets = 16;   // max terms (incl. the distance term) per problem
 
 // =============================================================================================
@@ -310,6 +313,94 @@ __global__ void __launch_bounds__(kThreads, 6) k_spmv(SpmvArgs<T> a, RedScratch 
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Wide Q (nd > kMaxDiag: custom operators): single GPU, CDS arrays only.  The offsets stay in device memory (every
+// thread of a warp reads the same one: a broadcast) and nothing is sized by nd, so any width works.  Each row
+// evaluates the expression of spmv_rows_vec / spmv_row_scalar in the array form, acc = acc + q_j * x[r + off_j] for
+// j = 0..nd-1 in Q_offsets order: the result is bit-identical to k_spmv on the same matrix.
+// ---------------------------------------------------------------------------------------------
+template <typename T>
+struct SpmvWideArgs {
+  const T* R;          // [nd][ld] diagonals, row aligned, zero padded
+  i64 ld;
+  int nd;
+  const i64* off;      // [nd] offsets in accumulation order (device memory)
+  i64 N;
+  const T* x;
+  T* y;
+};
+
+template <typename T>
+__device__ __forceinline__ void spmv_rows_wide(const SpmvWideArgs<T>& a, i64 r, T (&acc)[Vec<T>::W]) {
+  constexpr int VW = Vec<T>::W;
+#pragma unroll
+  for (int e = 0; e < VW; ++e) acc[e] = (T)0;
+#pragma unroll 4
+  for (int j = 0; j < a.nd; ++j) {
+    T rv[VW], xv[VW];
+    vload_stream<T>(a.R + (i64)j * a.ld + r, rv);
+    const i64 o = __ldg(a.off + j);
+    const i64 li = r + o;
+    if (li >= 0 && li + VW <= a.N) {
+      const T* xp = a.x + li;
+      if ((o & (VW - 1)) == 0) {
+        vload<T>(xp, xv);
+      } else {
+#pragma unroll
+        for (int e = 0; e < VW; ++e) xv[e] = xp[e];
+      }
+    } else {
+#pragma unroll
+      for (int e = 0; e < VW; ++e) {
+        const i64 ge = li + e;
+        xv[e] = (ge >= 0 && ge < a.N) ? a.x[ge] : (T)0;
+      }
+    }
+#pragma unroll
+    for (int e = 0; e < VW; ++e) acc[e] = acc[e] + rv[e] * xv[e];
+  }
+}
+
+template <typename T>
+__device__ __forceinline__ T spmv_row_wide_scalar(const SpmvWideArgs<T>& a, i64 r) {
+  T acc = (T)0;
+  for (int j = 0; j < a.nd; ++j) {
+    const i64 gc = r + __ldg(a.off + j);
+    if (gc >= 0 && gc < a.N) acc = acc + a.R[(i64)j * a.ld + r] * a.x[gc];
+  }
+  return acc;
+}
+
+// y = Q x and (DOT) the partial sum of x.*y -> out_dot[0]              (as k_spmv on one GPU)
+template <typename T, bool DOT>
+__global__ void __launch_bounds__(kThreads) k_spmv_wide(SpmvWideArgs<T> a, RedScratch rs, double* out_dot,
+                                                        const int* done_flag) {
+  if (done_flag && *done_flag) return;
+  constexpr int VW = Vec<T>::W;
+  double d[1] = {0.0};
+  const i64 nvec = a.N / VW;
+  for (i64 iv = (i64)blockIdx.x * blockDim.x + threadIdx.x; iv < nvec; iv += (i64)gridDim.x * blockDim.x) {
+    const i64 r = iv * VW;
+    T acc[VW];
+    spmv_rows_wide<T>(a, r, acc);
+    vstore<T>(a.y + r, acc);
+    if (DOT) {
+      T xc[VW];
+      vload<T>(a.x + r, xc);
+#pragma unroll
+      for (int e = 0; e < VW; ++e) d[0] += (double)xc[e] * (double)acc[e];
+    }
+  }
+  for (i64 r = nvec * VW + (i64)blockIdx.x * blockDim.x + threadIdx.x; r < a.N; r += (i64)gridDim.x * blockDim.x) {
+    const T acc = spmv_row_wide_scalar<T>(a, r);
+    a.y[r] = acc;
+    if (DOT) d[0] += (double)a.x[r] * (double)acc;
+  }
+  if (DOT) {
+    if (grid_sum<1>(d, rs) && threadIdx.x == 0) out_dot[0] = d[0];
+  }
+}
+
 // =============================================================================================
 // CG (device-resident scalars; the host only polls `done`)
 // =============================================================================================
@@ -388,6 +479,50 @@ __global__ void __launch_bounds__(kThreads) k_cg_init(SpmvArgs<T> a, const T* __
       st->bb = d[0];
       st->rr = d[1];
     }
+  }
+}
+
+// k_cg_init for a wide Q (single GPU): r = b - Q x ; p = r ; (x_old = x) ; sums bb, rr
+template <typename T>
+__global__ void __launch_bounds__(kThreads) k_cg_init_wide(SpmvWideArgs<T> a, const T* __restrict__ b, T* __restrict__ r,
+                                                           T* __restrict__ p, T* __restrict__ x_old, RedScratch rs,
+                                                           CgState* st) {
+  constexpr int VW = Vec<T>::W;
+  double d[2] = {0.0, 0.0};
+  const i64 nvec = a.N / VW;
+  for (i64 iv = (i64)blockIdx.x * blockDim.x + threadIdx.x; iv < nvec; iv += (i64)gridDim.x * blockDim.x) {
+    const i64 row = iv * VW;
+    T acc[VW], bv[VW], rv[VW];
+    spmv_rows_wide<T>(a, row, acc);
+    vload_stream<T>(b + row, bv);
+#pragma unroll
+    for (int e = 0; e < VW; ++e) {
+      rv[e] = bv[e] - acc[e];
+      d[0] += (double)bv[e] * (double)bv[e];
+      d[1] += (double)rv[e] * (double)rv[e];
+    }
+    vstore<T>(r + row, rv);
+    vstore<T>(p + row, rv);
+    if (x_old) {
+      T xc[VW];
+      vload<T>(a.x + row, xc);
+      vstore<T>(x_old + row, xc);
+    }
+  }
+  for (i64 row = nvec * VW + (i64)blockIdx.x * blockDim.x + threadIdx.x; row < a.N;
+       row += (i64)gridDim.x * blockDim.x) {
+    const T acc = spmv_row_wide_scalar<T>(a, row);
+    const T bv = b[row];
+    const T rv = bv - acc;
+    d[0] += (double)bv * (double)bv;
+    d[1] += (double)rv * (double)rv;
+    r[row] = rv;
+    p[row] = rv;
+    if (x_old) x_old[row] = a.x[row];
+  }
+  if (grid_sum<2>(d, rs) && threadIdx.x == 0) {
+    st->bb = d[0];
+    st->rr = d[1];
   }
 }
 
@@ -715,41 +850,67 @@ template <typename T>
 struct SparseRef {
   const long long* rp; const int* ci; const T* va;     // CSR of A
   const long long* cp; const int* ri; const T* vt;     // CSC of A
-  i64 rows, cols;
+  i64 rows, cols;                                      // of A (the block operator B has 2*cols columns unless PLAIN)
+  int mode;                                            // SIPB_BLOCK_*: B = A, [A 0], [0 A] or [A A]
 };
-// s = A x                                                     (update_y_l.jl:43, PARSDMM_initialize.jl:97)
+// columns of B
+template <typename T>
+__device__ __forceinline__ i64 sparse_block_cols(const SparseRef<T>& A) {
+  return A.mode == SIPB_BLOCK_PLAIN ? A.cols : 2 * A.cols;
+}
+// s = B x                                                     (update_y_l.jl:43, PARSDMM_initialize.jl:97)
+// SparseArrays' fold over row r of the hcat matrix: [A 0] and [0 A] fold over x[0:N) or x[N:2N); [A A] is ONE fold,
+// A's entries of the row on x[0:N) first, then the same entries on x[N:2N)  (not A x1 + A x2)
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_sparse_forward(SparseRef<T> A, const T* __restrict__ x, T* __restrict__ s) {
+  const T* x1 = A.mode == SIPB_BLOCK_RIGHT ? x + A.cols : x;
   for (i64 r = (i64)blockIdx.x * blockDim.x + threadIdx.x; r < A.rows; r += (i64)gridDim.x * blockDim.x) {
     T acc = (T)0;
-    for (long long q = A.rp[r]; q < A.rp[r + 1]; ++q) acc = acc + A.va[q] * x[A.ci[q]];
+    for (long long q = A.rp[r]; q < A.rp[r + 1]; ++q) acc = acc + A.va[q] * x1[A.ci[q]];
+    if (A.mode == SIPB_BLOCK_BOTH)
+      for (long long q = A.rp[r]; q < A.rp[r + 1]; ++q) acc = acc + A.va[q] * x[A.cols + A.ci[q]];
     s[r] = acc;
   }
 }
-// t = [t +] A' v  with  v = rho*y + l  (l == null: v = y)          (rhs_compose.jl:28-30)
+// column c of B: the column of A it holds, or -1 in a half B does not touch (there B' v is a fold over no entries: +0)
+template <typename T>
+__device__ __forceinline__ i64 sparse_block_col(const SparseRef<T>& A, i64 c) {
+  const bool upper = c >= A.cols;
+  return op_touches_half(A.mode, upper) ? (upper ? c - A.cols : c) : (i64)-1;
+}
+// t = [t +] B' v  with  v = rho*y + l  (l == null: v = y)          (rhs_compose.jl:28-30)
+// accumulate: t[c] + (B'v)[c], the expression of k_rhs (a +0 from an untouched half turns a -0 of t into +0 there too)
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_sparse_adjoint(SparseRef<T> A, T rho, const T* __restrict__ y,
                                                              const T* __restrict__ l, T* __restrict__ t, int accumulate) {
-  for (i64 c = (i64)blockIdx.x * blockDim.x + threadIdx.x; c < A.cols; c += (i64)gridDim.x * blockDim.x) {
+  const i64 ncols = sparse_block_cols<T>(A);
+  for (i64 c = (i64)blockIdx.x * blockDim.x + threadIdx.x; c < ncols; c += (i64)gridDim.x * blockDim.x) {
+    const i64 ca = sparse_block_col<T>(A, c);
     T acc = (T)0;
-    for (long long q = A.cp[c]; q < A.cp[c + 1]; ++q) {
-      const int r = A.ri[q];
-      const T v = l ? rho * y[r] + l[r] : y[r];
-      acc = acc + A.vt[q] * v;
+    if (ca >= 0) {
+      for (long long q = A.cp[ca]; q < A.cp[ca + 1]; ++q) {
+        const int r = A.ri[q];
+        const T v = l ? rho * y[r] + l[r] : y[r];
+        acc = acc + A.vt[q] * v;
+      }
     }
     t[c] = accumulate ? t[c] + acc : acc;
   }
 }
-// || A' (y - y_old) ||^2 -> out[0]                                 (update_y_l.jl:82-84)
+// || B' (y - y_old) ||^2 -> out[0]                                 (update_y_l.jl:82-84)
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_sparse_rdual(SparseRef<T> A, const T* __restrict__ y,
                                                            const T* __restrict__ y_old, RedScratch rs, double* out) {
   double d[1] = {0.0};
-  for (i64 c = (i64)blockIdx.x * blockDim.x + threadIdx.x; c < A.cols; c += (i64)gridDim.x * blockDim.x) {
+  const i64 ncols = sparse_block_cols<T>(A);
+  for (i64 c = (i64)blockIdx.x * blockDim.x + threadIdx.x; c < ncols; c += (i64)gridDim.x * blockDim.x) {
+    const i64 ca = sparse_block_col<T>(A, c);
     T acc = (T)0;
-    for (long long q = A.cp[c]; q < A.cp[c + 1]; ++q) {
-      const int r = A.ri[q];
-      acc = acc + A.vt[q] * (y[r] - y_old[r]);
+    if (ca >= 0) {
+      for (long long q = A.cp[ca]; q < A.cp[ca + 1]; ++q) {
+        const int r = A.ri[q];
+        acc = acc + A.vt[q] * (y[r] - y_old[r]);
+      }
     }
     d[0] += (double)acc * (double)acc;
   }
@@ -1314,6 +1475,31 @@ __global__ void __launch_bounds__(kThreads) k_cds_axpy(i64 N, T* __restrict__ A,
   }
   for (i64 r = nvec * VW + (i64)blockIdx.x * blockDim.x + threadIdx.x; r < N; r += (i64)gridDim.x * blockDim.x)
     A[r] = A[r] + alpha * B[r];
+}
+
+// Q[:, qcol[k]] += alpha * B[:, k] for k = 0..nd-1 in one launch (the Q update of a set whose A'A has more than
+// kMaxDiag diagonals; the columns qcol[] are distinct, so blockIdx.y-strided diagonals never write the same entry)
+template <typename T>
+__global__ void __launch_bounds__(kThreads) k_cds_axpy_wide(i64 N, i64 ld, int nd, T* __restrict__ Q,
+                                                            const int* __restrict__ qcol, const T* __restrict__ B,
+                                                            T alpha) {
+  constexpr int VW = Vec<T>::W;
+  const i64 nvec = N / VW;
+  for (int k = blockIdx.y; k < nd; k += gridDim.y) {
+    T* A = Q + (i64)__ldg(qcol + k) * ld;
+    const T* Bk = B + (i64)k * ld;
+    for (i64 iv = (i64)blockIdx.x * blockDim.x + threadIdx.x; iv < nvec; iv += (i64)gridDim.x * blockDim.x) {
+      const i64 r = iv * VW;
+      T av[VW], bv[VW];
+      vload<T>(A + r, av);
+      vload_stream<T>(Bk + r, bv);
+#pragma unroll
+      for (int e = 0; e < VW; ++e) av[e] = av[e] + alpha * bv[e];
+      vstore<T>(A + r, av);
+    }
+    for (i64 r = nvec * VW + (i64)blockIdx.x * blockDim.x + threadIdx.x; r < N; r += (i64)gridDim.x * blockDim.x)
+      A[r] = A[r] + alpha * Bk[r];
+  }
 }
 
 // ---- stencil-class tables (see RowClass above) ------------------------------------------------------------

@@ -763,11 +763,13 @@ struct SparseDev {
     return SIPB_OK;
   }
   i64 rows = 0, cols = 0;
-  SparseRef<T> ref() const {
+  // block_mode: the operator B the kernels apply, A itself or (Minkowski) [A 0], [0 A], [A A]
+  SparseRef<T> ref(int block_mode = SIPB_BLOCK_PLAIN) const {
     SparseRef<T> r;
     r.rp = rp.p; r.ci = ci.p; r.va = va.p;
     r.cp = cp.p; r.ri = ri.p; r.vt = vt.p;
     r.rows = rows; r.cols = cols;
+    r.mode = block_mode;
     return r;
   }
 };
@@ -1130,6 +1132,7 @@ struct SetT {
   int nd = 0;
   std::vector<int64_t> offs;
   std::vector<int> qcol;      // column of Q for each diagonal of AtA
+  DevBuf<int> qcol_d;         // nd > kMaxDiag: qcol on the device (k_cds_axpy_wide)
   bool has_ata = false;
   bool tab_direct = false;    // ata_tab came from the host (sipb_problem_set_ata_classes): nothing to extract / verify
   DevBuf<ProjParams<T>> pp_y, pp_f;   // dynamic projector parameters: y-update / feasibility
@@ -1151,6 +1154,8 @@ struct Problem : sipb_problem {
   i64 ld;                     // leading dimension of CDS arrays
   std::vector<std::unique_ptr<SetT<T>>> sets;
   std::vector<int64_t> q_offs;
+  DevBuf<i64> q_offs_d;     // wide Q (more than kMaxDiag diagonals): the offsets on the device (k_spmv_wide)
+  bool q_wide = false;
   DevBuf<T> Q, x, x_old, rhs, r, pvec, Ap, m, tmp;
   DevBuf<T> Q_tab;            // [kMaxClasses][nq] stencil-class form of Q (replaces Q when q_classes)
   bool q_classes = false;
@@ -1309,9 +1314,9 @@ struct Problem : sipb_problem {
     S->desc.sparse = nullptr;        // the host arrays are not kept
     int rc;
     if (d->op_kind == SIPB_OP_SPARSE) {
-      // custom_TD_OP (setup_constraints.jl:70-72): an explicit sparse matrix with N columns
-      SIPB_REQUIRE(!sg.on && !minkowski && !fiber, SIPB_E_UNSUPPORTED,
-                   "explicit sparse operators are single-GPU, non-Minkowski, matrix/tensor mode");
+      // custom_TD_OP (setup_constraints.jl:70-72): an explicit sparse matrix A with N columns; in a Minkowski problem the
+      // set's operator is [A 0], [0 A] or [A A] by block_mode (PARSDMM_precompute_distribute_Minkowski.jl:78-88)
+      SIPB_REQUIRE(!sg.on && !fiber, SIPB_E_UNSUPPORTED, "explicit sparse operators are single-GPU, matrix/tensor mode");
       SIPB_REQUIRE(d->sparse && d->sparse->cols == npts, SIPB_E_INVALID, "sparse operator must have prod(n) columns");
       rc = S->sparse.upload(d->sparse, ctx->stream);
       if (rc) return rc;
@@ -1369,7 +1374,7 @@ struct Problem : sipb_problem {
     SIPB_REQUIRE(!finalized, SIPB_E_STATE, "problem already finalized");
     SIPB_REQUIRE(idx >= 0 && idx < (int)sets.size(), SIPB_E_INVALID, "set index out of range");
     SIPB_REQUIRE(rows == N, SIPB_E_INVALID, "AtA must have N rows");
-    SIPB_REQUIRE(nd >= 1 && nd <= kMaxDiag, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,32]");
+    SIPB_REQUIRE(nd >= 1 && nd <= kMaxDiagWide, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,999]");
     SetT<T>& S = *sets[idx];
     SIPB_CUDA_CHECK(S.ata.alloc((size_t)ld * nd));
     SIPB_CUDA_CHECK(cudaMemsetAsync(S.ata.p, 0, (size_t)ld * nd * sizeof(T), ctx->stream));
@@ -1418,9 +1423,11 @@ struct Problem : sipb_problem {
     SIPB_REQUIRE(sets.size() <= 99, SIPB_E_UNSUPPORTED, "more than 99 operators");
     for (size_t i = 0; i < sets.size(); ++i) {
       for (int64_t o : sets[i]->offs) push_unique(o);
-      push_unique(0);   // padding zeros of column i (every column is padded: nd <= 32 < 999)
+      if (sets[i]->nd < kMaxDiagWide) push_unique(0);   // padding zeros of column i (a full column of 999 has none)
     }
-    SIPB_REQUIRE((int)q_offs.size() <= kMaxDiag, SIPB_E_UNSUPPORTED, "Q has more than 32 diagonals");
+    // more than kMaxDiag diagonals (custom operators): the *_wide kernels, CDS arrays, one GPU
+    q_wide = (int)q_offs.size() > kMaxDiag;
+    SIPB_REQUIRE(!(q_wide && sg.on), SIPB_E_UNSUPPORTED, "Q with more than 32 diagonals is single-GPU");
     for (auto& S : sets) {
       S->qcol.resize(S->nd);
       for (int k = 0; k < S->nd; ++k) {
@@ -1428,6 +1435,17 @@ struct Problem : sipb_problem {
         SIPB_REQUIRE(it != q_offs.end(), SIPB_E_MISSING_DIAG, "diagonal missing in Q");
         S->qcol[k] = (int)(it - q_offs.begin());
       }
+      if (S->nd > kMaxDiag) {
+        SIPB_CUDA_CHECK(S->qcol_d.alloc((size_t)S->nd));
+        SIPB_CUDA_CHECK(cudaMemcpyAsync(S->qcol_d.p, S->qcol.data(), S->nd * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+        SIPB_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+      }
+    }
+    if (q_wide) {
+      SIPB_CUDA_CHECK(q_offs_d.alloc(q_offs.size()));
+      SIPB_CUDA_CHECK(cudaMemcpyAsync(q_offs_d.p, q_offs.data(), q_offs.size() * sizeof(int64_t), cudaMemcpyHostToDevice,
+                                      ctx->stream));
+      SIPB_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
     }
     { int rc = detect_classes(); if (rc) return rc; }
     cudaError_t e = cudaSuccess;
@@ -1468,11 +1486,16 @@ struct Problem : sipb_problem {
     int ok = !(env && env[0] == '0');
     if (n[0] * n[1] * n[2] >= ((i64)1 << 31)) ok = 0;
     if (minkowski && sg.on) ok = 0;
+    // class tables hold at most kMaxDiag diagonals: a wide Q (or A'A) stays in array form
+    bool wide = q_wide;
+    for (auto& S : sets) wide = wide || S->nd > kMaxDiag;
+    if (wide) ok = 0;
     sipb_ctx* c = ctx;
     bool any_direct = false, all_direct = true;
     for (auto& S : sets) { any_direct = any_direct || S->tab_direct; all_direct = all_direct && S->tab_direct; }
     if (any_direct) {
       // class tables handed over by the host: there is no array to fall back to
+      SIPB_REQUIRE(!wide, SIPB_E_UNSUPPORTED, "stencil-class tables hold at most 32 diagonals of Q");
       SIPB_REQUIRE(ok, SIPB_E_STATE, "stencil-class tables were passed although SIPB_Q_CLASSES=0 asks for CDS arrays");
       SIPB_REQUIRE(all_direct, SIPB_E_STATE,
                    "either every AtA comes as a stencil-class table or every AtA comes as a CDS array");
@@ -1525,6 +1548,9 @@ struct Problem : sipb_problem {
       const int cnt = kMaxClasses * S.nd;
       LAUNCH(c, KC_Q_UPDATE, k_class_axpy<T>, (cnt + kThreads - 1) / kThreads, Q_tab.p, (int)q_offs.size(),
              (const T*)S.ata_tab.p, S.nd, qc, alpha);
+    } else if (S.nd > kMaxDiag) {
+      const dim3 grid((unsigned)c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), (unsigned)std::min(S.nd, 65535));
+      LAUNCH(c, KC_Q_UPDATE, k_cds_axpy_wide<T>, grid, N, ld, S.nd, Q.p, (const int*)S.qcol_d.p, (const T*)S.ata.p, alpha);
     } else {
       const int gN = c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W);
       for (int k = 0; k < S.nd; ++k)
@@ -1701,6 +1727,13 @@ struct Problem : sipb_problem {
     }
     a.N = N; a.row0 = sg.on ? sg.plane * sg.k0 : 0; a.Nglob = Nglob; a.x = xin; a.y = yout;
     a.x_lo = nullptr; a.x_hi = nullptr; a.n_lo = 0;
+    return a;
+  }
+  // argument block of the wide kernels (q_wide)
+  SpmvWideArgs<T> spmv_wide_args(const T* xin, T* yout) const {
+    SpmvWideArgs<T> a;
+    a.R = Q.p; a.ld = ld; a.nd = (int)q_offs.size(); a.off = q_offs_d.p;
+    a.N = N; a.x = xin; a.y = yout;
     return a;
   }
   // SpMV on p with the neighbours' planes read through peer pointers
@@ -1982,10 +2015,13 @@ struct Problem : sipb_problem {
     // (k_cg_init measured faster with two waves than with one: 2.03 vs 2.68 ms per solve at 200^3)
     const int g_init = c->grid_for(nvecN), g_mv = c->grid_fit((const void*)k_spmv<T, true>, nvecN),
               g_xr = c->grid_fit((const void*)k_cg_xr<T>, nvecN), g_p = c->grid_fit((const void*)k_cg_p<T>, nvecN);
+    const int g_mv_wide = q_wide ? c->grid_fit((const void*)k_spmv_wide<T, true>, nvecN) : 0;
     const bool tiled = tile.ok && q_classes;
     // r = b - Qx, p = r, x_old = x, tolerance rule / early exits        (argmin_x.jl:33-37, cg.jl:47-76)
     auto launch_init = [&](const LoopCond& lc) -> int {
-      if (tiled) {
+      if (q_wide) {
+        LAUNCH(c, KC_CG_INIT, k_cg_init_wide<T>, g_init, spmv_wide_args(xv, nullptr), b, rr, pp, x_old_out, c->rs, c->d_cg);
+      } else if (tiled) {
         const TileInit<T> ti{b, rr, pp, x_old_out};
         if ((rc = launch_tile<T, 2>(c, KC_CG_INIT, tile, false, spmv_args(xv, nullptr), ti, nullptr, nullptr, c->d_cg, cd)))
           return rc;
@@ -2001,7 +2037,9 @@ struct Problem : sipb_problem {
     // one CG iteration                                                  (cg.jl:84-114)
     auto launch_iter = [&](const LoopCond& lc, const int* done_flag) -> int {
       if (!peer && (rc = exchange(pp, sg.nloc(), true, true))) return rc;     // halo planes of p
-      if (tiled) {
+      if (q_wide) {
+        LAUNCH(c, KC_SPMV_DOT, (k_spmv_wide<T, true>), g_mv_wide, spmv_wide_args(pp, Ap.p), c->rs, &c->d_cg->pAp, done_flag);
+      } else if (tiled) {
         const TileInit<T> ti{nullptr, nullptr, nullptr, nullptr};
         if ((rc = launch_tile<T, 1>(c, KC_SPMV_DOT, tile, false, spmv_args_peer(Ap.p), ti, &c->d_cg->pAp, done_flag, c->d_cg, cd)))
           return rc;
@@ -2172,7 +2210,7 @@ int Problem<T>::rhs_phase(int i, const std::vector<T>& rho, bool fuse_rdual) {
     while (s0 < p) {
       if (sets[s0]->is_sparse) {
         SetT<T>& S = *sets[s0];
-        LAUNCH(c, KC_RHS, k_sparse_adjoint<T>, c->grid_for(N), S.sparse.ref(), rho[s0], (const T*)S.y.p, (const T*)S.l.p,
+        LAUNCH(c, KC_RHS, k_sparse_adjoint<T>, c->grid_for(N), S.sparse.ref(S.desc.block_mode), rho[s0], (const T*)S.y.p, (const T*)S.l.p,
                rhs.p, first ? 0 : 1);
         first = false;
         ++s0;
@@ -2241,7 +2279,7 @@ int Problem<T>::yl_phase(int i, const std::vector<T>& rho, const std::vector<T>&
     ya.P = proj_static(S, rho[s]);
     ya.x = x.p; ya.y = S.y.p; ya.l = S.l.p; ya.y_old = S.y_old.p; ya.s = S.s.p;
     if (S.is_sparse) {       // s = A x by the sparse kernel; the fused kernels then apply the identity to it
-      LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(S.M), S.sparse.ref(), (const T*)x.p, S.s.p);
+      LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(S.M), S.sparse.ref(S.desc.block_mode), (const T*)x.p, S.s.p);
       ya.x = S.s.p;
     }
     ya.lhat0 = S.lhat0.p; ya.s0 = S.s0.p; ya.l0 = S.l0.p; ya.y0 = S.y0.p;
@@ -2326,7 +2364,7 @@ int Problem<T>::yl_phase(int i, const std::vector<T>& rho, const std::vector<T>&
     for (int s = 0; s < p; ++s) {
       SetT<T>& S = *sets[s];
       if (S.is_sparse)
-        LAUNCH(c, KC_RDUAL, k_sparse_rdual<T>, c->grid_for(N), S.sparse.ref(), (const T*)S.y.p, (const T*)S.y_old.p, c->rs,
+        LAUNCH(c, KC_RDUAL, k_sparse_rdual<T>, c->grid_for(N), S.sparse.ref(S.desc.block_mode), (const T*)S.y.p, (const T*)S.y_old.p, c->rs,
                c->d_scal + s * kSlotPerSet + 3);
       else
         LAUNCH(c, KC_RDUAL, k_rdual<T>, c->grid_for((npts + Vec<T>::W - 1) / Vec<T>::W), S.op, (const T*)S.y.p,
@@ -2423,7 +2461,7 @@ int Problem<T>::solve(const void* m_h, void* x_h, void* const* l_h, void* const*
   for (int i = 0; i < nP; ++i) {
     SetT<T>& S = *sets[i];
     T* sv = S.s.p ? S.s.p : tmp.p;    // element-wise sets do not keep s: use the scratch vector
-    if (S.is_sparse) LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(S.M), S.sparse.ref(), (const T*)m.p, sv);
+    if (S.is_sparse) LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(S.M), S.sparse.ref(S.desc.block_mode), (const T*)m.p, sv);
     else LAUNCH(c, KC_OP_APPLY, k_op_forward<T>, c->grid_for(S.M), S.op, (const T*)m.p, sv);
     int rc = feasibility_of(S, sv, i * kSlotPerSet + 1);
     if (rc) return rc;
@@ -3141,6 +3179,19 @@ static int cds_spmv_impl(sipb_ctx* c, int64_t N, int nd, const void* R, const in
   SIPB_CUDA_CHECK(dx.alloc((size_t)N));
   SIPB_CUDA_CHECK(dy.alloc((size_t)N));
   SIPB_CUDA_CHECK(cudaMemcpyAsync(dx.p, x, N * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+  if (nd > kMaxDiag) {         // wide matrix: offsets from device memory
+    DevBuf<i64> doff;
+    SIPB_CUDA_CHECK(doff.alloc((size_t)nd));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(doff.p, offs, nd * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    SpmvWideArgs<T> a;
+    a.R = dR.p; a.ld = ld; a.nd = nd; a.off = doff.p; a.N = N; a.x = dx.p; a.y = dy.p;
+    LAUNCH(c, KC_SPMV, (k_spmv_wide<T, false>), c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), a, c->rs, (double*)nullptr,
+           (const int*)nullptr);
+    SIPB_CUDA_CHECK(cudaGetLastError());
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(y, dy.p, N * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));
+    return SIPB_OK;
+  }
   SpmvArgs<T> a;
   a.R = dR.p; a.ld = ld; a.nd = nd;
   for (int j = 0; j < nd; ++j) a.off[j] = offs[j];
@@ -3165,6 +3216,11 @@ static int cds_cg_impl(sipb_ctx* c, int64_t N, int nd, const void* R, const int6
   int rc = upload_cds<T>(c, N, nd, R, P.ld, P.Q);
   if (rc) return rc;
   P.q_offs.assign(offs, offs + nd);
+  P.q_wide = nd > kMaxDiag;
+  if (P.q_wide) {
+    SIPB_CUDA_CHECK(P.q_offs_d.alloc((size_t)nd));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(P.q_offs_d.p, offs, nd * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+  }
   DevBuf<T> db;
   SIPB_CUDA_CHECK(db.alloc((size_t)N));
   SIPB_CUDA_CHECK(P.x.alloc((size_t)N));
@@ -3248,19 +3304,21 @@ static int op_apply_impl(sipb_ctx* c, int ndim, const int64_t* n, const double* 
 }
 
 template <typename T>
-static int sparse_apply_impl(sipb_ctx* c, const sipb_sparse* A, int adjoint, const void* in, void* out) {
+static int sparse_apply_impl(sipb_ctx* c, const sipb_sparse* A, int block_mode, int adjoint, const void* in, void* out) {
   SparseDev<T> sd;
   int rc = sd.upload(A, c->stream);
   if (rc) return rc;
-  const i64 nin = adjoint ? A->rows : A->cols, nout = adjoint ? A->cols : A->rows;
+  const i64 bcols = block_mode == SIPB_BLOCK_PLAIN ? A->cols : 2 * A->cols;      // columns of the block operator
+  const i64 nin = adjoint ? A->rows : bcols, nout = adjoint ? bcols : A->rows;
   DevBuf<T> di, dout;
   SIPB_CUDA_CHECK(di.alloc((size_t)nin));
   SIPB_CUDA_CHECK(dout.alloc((size_t)nout));
   SIPB_CUDA_CHECK(cudaMemcpyAsync(di.p, in, nin * sizeof(T), cudaMemcpyHostToDevice, c->stream));
   if (adjoint)
-    LAUNCH(c, KC_OP_APPLY, k_sparse_adjoint<T>, c->grid_for(nout), sd.ref(), (T)1, (const T*)di.p, (const T*)nullptr, dout.p, 0);
+    LAUNCH(c, KC_OP_APPLY, k_sparse_adjoint<T>, c->grid_for(nout), sd.ref(block_mode), (T)1, (const T*)di.p,
+           (const T*)nullptr, dout.p, 0);
   else
-    LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(nout), sd.ref(), (const T*)di.p, dout.p);
+    LAUNCH(c, KC_OP_APPLY, k_sparse_forward<T>, c->grid_for(nout), sd.ref(block_mode), (const T*)di.p, dout.p);
   SIPB_CUDA_CHECK(cudaGetLastError());
   SIPB_CUDA_CHECK(cudaMemcpyAsync(out, dout.p, nout * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
   SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));
@@ -3276,14 +3334,30 @@ static int cds_scaled_add_impl(sipb_ctx* c, int64_t N, int nd_a, void* A, const 
   if (rc) return rc;
   rc = upload_cds<T>(c, N, nd_b, B, ld, dB);
   if (rc) return rc;
+  std::vector<int> cols((size_t)nd_b);
   for (int k = 0; k < nd_b; ++k) {
     int col = -1;
     for (int j = 0; j < nd_a; ++j) if (a_off[j] == b_off[k]) { col = j; break; }
     SIPB_REQUIRE(col >= 0, SIPB_E_MISSING_DIAG,
                  "attempted to update a diagonal in A in CDS storage that does not exist. A and B need to have the "
                  "same nonzero diagonals");
-    LAUNCH(c, KC_Q_UPDATE, k_cds_axpy<T>, c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), N, dA.p + (size_t)col * ld,
-           (const T*)(dB.p + (size_t)k * ld), (T)alpha);
+    cols[k] = col;
+  }
+  if (nd_b > kMaxDiag) {       // all diagonals of B in one launch, as the solver's Q update of a wide A'A
+    std::vector<int> sorted(cols);
+    std::sort(sorted.begin(), sorted.end());
+    SIPB_REQUIRE(std::adjacent_find(sorted.begin(), sorted.end()) == sorted.end(), SIPB_E_INVALID,
+                 "the offsets of B must be distinct");
+    DevBuf<int> dcol;
+    SIPB_CUDA_CHECK(dcol.alloc((size_t)nd_b));
+    SIPB_CUDA_CHECK(cudaMemcpyAsync(dcol.p, cols.data(), nd_b * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    const dim3 grid((unsigned)c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), (unsigned)std::min(nd_b, 65535));
+    LAUNCH(c, KC_Q_UPDATE, k_cds_axpy_wide<T>, grid, N, ld, nd_b, dA.p, (const int*)dcol.p, (const T*)dB.p, (T)alpha);
+    SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));     // dcol is released at the end of this scope
+  } else {
+    for (int k = 0; k < nd_b; ++k)
+      LAUNCH(c, KC_Q_UPDATE, k_cds_axpy<T>, c->grid_for((N + Vec<T>::W - 1) / Vec<T>::W), N, dA.p + (size_t)cols[k] * ld,
+             (const T*)(dB.p + (size_t)k * ld), (T)alpha);
   }
   SIPB_CUDA_CHECK(cudaGetLastError());
   SIPB_CUDA_CHECK(cudaMemcpy2DAsync(A, N * sizeof(T), dA.p, ld * sizeof(T), N * sizeof(T), nd_a, cudaMemcpyDeviceToHost,
@@ -3574,12 +3648,65 @@ static int iter_probe_impl(Problem<T>* P, int it, int do_adapt, const void* m_h,
   return SIPB_OK;
 }
 
+// form 2: the wide SpMV + dot (k_spmv_wide) on CDS arrays with the 125 diagonals of the A'A of a 3-D 27-point stencil
+// (the 5 x 5 x 5 box of offsets), 0 first and the others in box order, as Q_offsets would list them
+template <typename T>
+static int bench_spmv_wide(sipb_ctx* c, int ndim, const int64_t* n, int warmup, int reps, int flush_l2, double* avg_ms,
+                           int64_t* alg_bytes) {
+  SIPB_REQUIRE(ndim == 3, SIPB_E_INVALID, "the wide SpMV benchmark runs on a 3-D grid");
+  const i64 N = n[0] * n[1] * n[2];
+  const i64 ld = (N + 63) / 64 * 64;
+  std::vector<i64> offs{0};
+  for (int dk = -2; dk <= 2; ++dk)
+    for (int dj = -2; dj <= 2; ++dj)
+      for (int di = -2; di <= 2; ++di)
+        if (di || dj || dk) offs.push_back(di + n[0] * (dj + n[1] * dk));
+  const int nd = (int)offs.size();
+  DevBuf<T> dR, dx, dy, flush;
+  DevBuf<i64> doff;
+  SIPB_CUDA_CHECK(dR.alloc((size_t)ld * nd));
+  SIPB_CUDA_CHECK(dx.alloc((size_t)N));
+  SIPB_CUDA_CHECK(dy.alloc((size_t)N));
+  SIPB_CUDA_CHECK(doff.alloc((size_t)nd));
+  SIPB_CUDA_CHECK(cudaMemcpyAsync(doff.p, offs.data(), nd * sizeof(i64), cudaMemcpyHostToDevice, c->stream));
+  const size_t flush_elems = (size_t)(256u << 20) / sizeof(T);
+  if (flush_l2) SIPB_CUDA_CHECK(flush.alloc(flush_elems));
+  LAUNCH(c, KC_FILL, k_fill<T>, c->max_grid(), (i64)ld * nd, dR.p, (T)0.25);
+  LAUNCH(c, KC_FILL, k_fill<T>, c->max_grid(), N, dx.p, (T)1.5);
+  SpmvWideArgs<T> a;
+  a.R = dR.p; a.ld = ld; a.nd = nd; a.off = doff.p; a.N = N; a.x = dx.p; a.y = dy.p;
+  const int g = c->grid_fit((const void*)k_spmv_wide<T, true>, (N + Vec<T>::W - 1) / Vec<T>::W);
+  cudaEvent_t e0, e1;
+  SIPB_CUDA_CHECK(cudaEventCreate(&e0));
+  SIPB_CUDA_CHECK(cudaEventCreate(&e1));
+  double total = 0.0;
+  for (int it = 0; it < warmup + reps; ++it) {
+    if (flush_l2) LAUNCH(c, KC_FILL, k_fill<T>, c->max_grid(), (i64)flush_elems, flush.p, (T)it);
+    SIPB_CUDA_CHECK(cudaEventRecord(e0, c->stream));
+    LAUNCH(c, KC_SPMV_DOT, (k_spmv_wide<T, true>), g, a, c->rs, c->d_scal, (const int*)nullptr);
+    SIPB_CUDA_CHECK(cudaEventRecord(e1, c->stream));
+    SIPB_CUDA_CHECK(cudaEventSynchronize(e1));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, e0, e1);
+    if (it >= warmup) total += ms;
+  }
+  cudaEventDestroy(e0);
+  cudaEventDestroy(e1);
+  SIPB_CUDA_CHECK(cudaGetLastError());
+  SIPB_CUDA_CHECK(cudaMemsetAsync(c->d_scal, 0, sizeof(double), c->stream));
+  SIPB_CUDA_CHECK(cudaStreamSynchronize(c->stream));
+  *avg_ms = total / std::max(1, reps);
+  *alg_bytes = (int64_t)(nd + 2) * N * (int64_t)sizeof(T);
+  return SIPB_OK;
+}
+
 template <typename T>
 static int bench_spmv_impl(sipb_ctx* c, int ndim, const int64_t* n, int warmup, int reps, int flush_l2, double* avg_ms,
                            int64_t* alg_bytes, int form, int tiled) {
   const i64 N = n[0] * n[1] * (ndim == 3 ? n[2] : 1);
   const i64 ld = (N + 63) / 64 * 64;
   std::vector<int64_t> offs;
+  if (form == 2) return bench_spmv_wide<T>(c, ndim, n, warmup, reps, flush_l2, avg_ms, alg_bytes);
   // Q_offsets of bounds/identity + TV + distance in the reference's order: [0, -n1n2, -n1, -1, 1, n1, n1n2]
   offs.push_back(0);
   if (ndim == 3) offs.push_back(-n[0] * n[1]);
@@ -3658,14 +3785,14 @@ extern "C" {
 int sipb_cds_spmv(sipb_ctx* ctx, int dtype, int64_t N, int nd, const void* R, const int64_t* offsets, const void* x,
                   void* y) {
   SIPB_REQUIRE(ctx && R && offsets && x && y, SIPB_E_INVALID, "null argument");
-  SIPB_REQUIRE(nd >= 1 && nd <= kMaxDiag, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,32]");
+  SIPB_REQUIRE(nd >= 1 && nd <= kMaxDiagWide, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,999]");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
   DISPATCH(dtype, cds_spmv_impl, ctx, N, nd, R, offsets, x, y);
 }
 int sipb_cds_cg(sipb_ctx* ctx, int dtype, int64_t N, int nd, const void* R, const int64_t* offsets, const void* b,
                 void* x, double tol, int max_iter, int* flag, double* relres, int* iters) {
   SIPB_REQUIRE(ctx && R && offsets && b && x && flag && relres && iters, SIPB_E_INVALID, "null argument");
-  SIPB_REQUIRE(nd >= 1 && nd <= kMaxDiag, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,32]");
+  SIPB_REQUIRE(nd >= 1 && nd <= kMaxDiagWide, SIPB_E_UNSUPPORTED, "number of diagonals outside [1,999]");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
   DISPATCH(dtype, cds_cg_impl, ctx, N, nd, R, offsets, b, x, tol, max_iter, flag, relres, iters);
 }
@@ -3691,11 +3818,19 @@ int sipb_op_apply(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, const do
 int sipb_sparse_apply(sipb_ctx* ctx, int dtype, const sipb_sparse* A, int adjoint, const void* in, void* out) {
   SIPB_REQUIRE(ctx && A && in && out, SIPB_E_INVALID, "null argument");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
-  DISPATCH(dtype, sparse_apply_impl, ctx, A, adjoint, in, out);
+  DISPATCH(dtype, sparse_apply_impl, ctx, A, SIPB_BLOCK_PLAIN, adjoint, in, out);
+}
+int sipb_sparse_apply_block(sipb_ctx* ctx, int dtype, const sipb_sparse* A, int block_mode, int adjoint, const void* in,
+                            void* out) {
+  SIPB_REQUIRE(ctx && A && in && out, SIPB_E_INVALID, "null argument");
+  SIPB_REQUIRE(block_mode >= SIPB_BLOCK_PLAIN && block_mode <= SIPB_BLOCK_BOTH, SIPB_E_INVALID, "unknown block_mode");
+  SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
+  DISPATCH(dtype, sparse_apply_impl, ctx, A, block_mode, adjoint, in, out);
 }
 int sipb_cds_scaled_add(sipb_ctx* ctx, int dtype, int64_t N, int nd_a, void* A, const int64_t* a_offsets, int nd_b,
                         const void* B, const int64_t* b_offsets, double alpha) {
   SIPB_REQUIRE(ctx && A && a_offsets && B && b_offsets, SIPB_E_INVALID, "null argument");
+  SIPB_REQUIRE(nd_b <= kMaxDiagWide, SIPB_E_UNSUPPORTED, "B has more than 999 diagonals");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
   DISPATCH(dtype, cds_scaled_add_impl, ctx, N, nd_a, A, a_offsets, nd_b, B, b_offsets, alpha);
 }
@@ -3708,7 +3843,8 @@ int sipb_bench_spmv(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, int wa
 int sipb_bench_spmv2(sipb_ctx* ctx, int dtype, int ndim, const int64_t* n, int warmup, int reps, int flush_l2, int form,
                      int tiled, double* avg_ms, int64_t* algorithmic_bytes) {
   SIPB_REQUIRE(ctx && n && avg_ms && algorithmic_bytes, SIPB_E_INVALID, "null argument");
-  SIPB_REQUIRE(form == 0 || form == 1, SIPB_E_INVALID, "form must be 0 (CDS arrays) or 1 (stencil classes)");
+  SIPB_REQUIRE(form >= 0 && form <= 2, SIPB_E_INVALID,
+               "form must be 0 (CDS arrays), 1 (stencil classes) or 2 (125 diagonals, wide kernel)");
   SIPB_CUDA_CHECK(cudaSetDevice(ctx->device));
   DISPATCH(dtype, bench_spmv_impl, ctx, ndim, n, warmup, reps, flush_l2, avg_ms, algorithmic_bytes, form, tiled);
 }

@@ -12,6 +12,7 @@ light `TDOperator` descriptor (kind, grid, spacing) that
 """
 from __future__ import annotations
 
+import copy
 import ctypes as C
 
 import numpy as np
@@ -283,7 +284,8 @@ class SparseOperator(TDOperator):
     (setup_constraints.jl:70-72, examples/ConstraintSetupExamples.jl:125-146).  Held on the host as a SciPy CSC
     matrix (the SparseMatrixCSC of the reference); the device gets CSR and CSC copies and applies them with
     SparseArrays' fold order (ascending column inside a row, ascending row inside a column).
-    Single GPU, non-Minkowski, matrix/tensor mode."""
+    Inside a generalized Minkowski set `with_block` gives [A 0], [0 A] or [A A]; the device applies the block form
+    without forming it.  Single GPU, matrix/tensor mode."""
 
     def __init__(self, A, n, h, TF):
         self.kind = "custom"
@@ -310,13 +312,27 @@ class SparseOperator(TDOperator):
         return self._sparse.shape[0]
 
     def with_block(self, block_mode):
-        raise NotImplementedError("custom operators inside generalized Minkowski sets are not on the device path")
+        """[A 0], [0 A] or [A A] (PARSDMM_precompute_distribute_Minkowski.jl:78-88): a copy with 2N columns that
+        shares A's host arrays; `tosparse()` of the copy is the hcat matrix."""
+        B = copy.copy(self)
+        B.block_mode = block_mode
+        B._block = None
+        return B
 
     def __repr__(self):
         return "SparseOperator(%dx%d, nnz=%d, %s)" % (*self.shape, self._sparse.nnz, self.TF.__name__)
 
     def tosparse(self) -> sp.csc_matrix:
-        return self._sparse
+        if self.block_mode == _lib.BLOCK_PLAIN:
+            return self._sparse
+        if getattr(self, "_block", None) is None:
+            A = self._sparse
+            Z = sp.csc_matrix(A.shape, dtype=self.TF)
+            B = sp.hstack({_lib.BLOCK_LEFT: [A, Z], _lib.BLOCK_RIGHT: [Z, A], _lib.BLOCK_BOTH: [A, A]}[self.block_mode],
+                          format="csc", dtype=self.TF)
+            B.sort_indices()
+            self._block = B
+        return self._block
 
     def sparse_struct(self) -> _lib.Sparse:
         """ctypes view (sipb_sparse) of the CSR + CSC arrays; the arrays stay alive with this object."""
@@ -342,18 +358,26 @@ class SparseOperator(TDOperator):
             raise ValueError("dimension mismatch: operator is %dx%d, vector has %d" % (*self.shape, v.size))
         out = np.empty(nout, dtype=self.TF)
         lib = _lib.load()
-        _lib.check(lib.sipb_sparse_apply(_lib.ctx(), _lib.dtype_code(self.TF), C.byref(self.sparse_struct()),
-                                         1 if adjoint else 0, v.ctypes.data, out.ctypes.data))
+        if self.block_mode == _lib.BLOCK_PLAIN:
+            _lib.check(lib.sipb_sparse_apply(_lib.ctx(), _lib.dtype_code(self.TF), C.byref(self.sparse_struct()),
+                                             1 if adjoint else 0, v.ctypes.data, out.ctypes.data))
+        else:
+            _lib.check(lib.sipb_sparse_apply_block(_lib.ctx(), _lib.dtype_code(self.TF), C.byref(self.sparse_struct()),
+                                                   self.block_mode, 1 if adjoint else 0, v.ctypes.data, out.ctypes.data))
         return out
 
     def ata_cds(self, zrange=None):
-        """mat2CDS(A'*A) (PARSDMM_precompute_distribute.jl:47,52-55)."""
+        """mat2CDS(A'*A) (PARSDMM_precompute_distribute.jl:47,52-55); for a block copy mat2CDS of the 2N x 2N block
+        matrix [A'A 0;0 0], [0 0;0 A'A] or [A'A A'A;A'A A'A] (PARSDMM_precompute_distribute_Minkowski.jl:32-74)."""
         if zrange is not None:
             raise NotImplementedError("custom operators are single-GPU (no slab decomposition)")
         A = self._sparse
         AtA = sp.csc_matrix(sp.csc_matrix(A.T) @ A).astype(self.TF)
         AtA.sort_indices()
-        return mat2CDS(AtA)
+        R, offs = mat2CDS(AtA)
+        if self.block_mode == _lib.BLOCK_PLAIN:
+            return R, offs
+        return _minkowski_cds(R, offs, self.block_mode)
 
 
 class _Adjoint:

@@ -70,11 +70,27 @@ def _classes_enabled() -> bool:
     return os.environ.get("SIPB_Q_CLASSES", "1") != "0"
 
 
+MAX_ATA_DIAGONALS = 999     # per A'A: the 999 x 99 offset table of PARSDMM_initialize.jl:217-221
+
+
 def _require_device_operators(TD_OP):
     for A in TD_OP:
         if not isinstance(A, TDOperator):
             raise NotImplementedError("only the banded operators built by get_TD_operator are on the device path; "
                                       "got %r" % type(A))
+
+
+def _require_banded_custom(set_Prop, i):
+    # custom operator: the caller describes it through set_Prop (ConstraintSetupExamples.jl:114-117)
+    if not set_Prop.banded[i] or set_Prop.dense[i]:
+        raise NotImplementedError("custom operators must be flagged banded and not dense: the device path solves "
+                                  "the x-subproblem in compressed-diagonal storage only")
+
+
+def _require_width(offs):
+    if offs.size > MAX_ATA_DIAGONALS:
+        raise NotImplementedError("A'A of the custom operator has %d diagonals; the reference's offset table holds %d"
+                                  % (offs.size, MAX_ATA_DIAGONALS))
 
 
 def PARSDMM_precompute_distribute(TD_OP, set_Prop, comp_grid, options):
@@ -103,16 +119,12 @@ def PARSDMM_precompute_distribute(TD_OP, set_Prop, comp_grid, options):
         AtA.slab = zrange
     for i in range(p):
         if isinstance(TD_OP[i], SparseOperator):
-            # custom operator: the caller describes it through set_Prop (ConstraintSetupExamples.jl:114-117)
-            if not set_Prop.banded[i] or set_Prop.dense[i]:
-                raise NotImplementedError("custom operators must be flagged banded and not dense: the device path solves "
-                                          "the x-subproblem in compressed-diagonal storage only")
+            _require_banded_custom(set_Prop, i)
             if set_Prop.AtA_diag[i]:          # :44-45: AtA = I when the caller says A'A is the identity
                 R, offs = np.ones((TD_OP[i].cols, 1), dtype=TF, order="F"), np.array([0], dtype=np.int64)
             else:
                 R, offs = TD_OP[i].ata_cds(zrange)
-            if offs.size > 32:
-                raise NotImplementedError("A'A of the custom operator has %d diagonals; the device path handles 32" % offs.size)
+            _require_width(offs)
         else:
             ct = TD_OP[i].ata_class_table() if _classes_enabled() else None
             if ct is not None:       # == mat2CDS(TD_OP[i]'*TD_OP[i]), formed only when somebody indexes AtA[i]
@@ -164,11 +176,21 @@ def PARSDMM_precompute_distribute_Minkowski(TD_OP_c1, TD_OP_c2, TD_OP_sum, set_P
     TD_OP = list(TD_OP_c1) + list(TD_OP_c2) + list(TD_OP_sum)
     s = len(TD_OP)
     AtA = CDSList()
+    # stencil-class tables for every set or CDS arrays for every set: a custom operator has no table
+    custom = any(isinstance(A, SparseOperator) for A in TD_OP)
     for i in range(s):
-        ct = TD_OP[i].ata_class_table() if _classes_enabled() and not isinstance(TD_OP[i], SparseOperator) else None
+        ct = TD_OP[i].ata_class_table() if _classes_enabled() and not custom else None
         if ct is not None:
             AtA.append_lazy(TD_OP[i], None)
             set_Prop.AtA_offsets[i] = ct[1]
+            continue
+        if isinstance(TD_OP[i], SparseOperator):
+            # mat2CDS of the block matrix of A'A (:32-74); its AtA_diag flag only matters for dense operators
+            _require_banded_custom(set_Prop, i)
+            R, offs = TD_OP[i].ata_cds()
+            _require_width(offs)
+            AtA.append(R)
+            set_Prop.AtA_offsets[i] = offs
             continue
         R, offs = TD_OP[i].ata_cds()
         AtA.append(R)
